@@ -12,6 +12,7 @@ pairs (no data-path collective), so scaling is weak and 8 GPUs x 128 pairs is th
   python bench.py --gpus N --steps K --warmup W            (torchrun for N > 1, one rank per GPU)
   python bench.py --impl reference ...                      the reference's CPU path (oracle port,
                                                             scipy ARPACK/SuperLU/cKDTree) on all host cores
+  python bench.py ... --dump-outputs DIR                    also write the last timed step's results to DIR/*.npy
 
 Prints ONE JSON line (rank 0).  `value` = pairs/s with the vertices already resident in HBM;
 `e2e` = the same through the public API from pinned host buffers with the result read back.
@@ -31,6 +32,11 @@ sys.path.insert(0, ROOT)
 
 NU = 39
 N_SPECTRAL, N_EXTRA, N_SAMPLES, SMOOTH_T, SMOOTH_S = 3, 3, 5000, 300, 40
+# --dump-outputs: the results of SpectralBatch.run that are written, and the number of vertices (per side) in the fixed
+# sample that per-vertex results are written for (128 pairs x 15 212 vertices in full would exceed 64 MB)
+DUMP_KEYS = ("eig_vals", "eig_vecs", "Q", "spectral_weights", "final_idx", "weighted_avg_transformed_points",
+             "nearest_neighbor_transformed_points")
+DUMP_ROWS = 1 << 17
 
 
 def make_pairs(pair_ids, nu=NU):
@@ -71,6 +77,34 @@ def config_dict(pairs_per_gpu, nu, n):
             "workload_pairs_per_gpu": pairs_per_gpu, "vertices_per_mesh": n,
             "l2": "GPU arm: working set >> L2 (batched CSR + blocks ~ %.1f GB per GPU), no flush needed; CPU arm: n/a"
                   % (pairs_per_gpu * 2 * 12e6 / 1e9)}
+
+
+def dump_outputs(outs, n_eig, out_dir):
+    """Write what one step returned -- `outs`: the DUMP_KEYS of SpectralBatch.run per sub-batch, sub-batches in pair
+    order -- to out_dir/<name>.npy, all float64.  Per-pair results are written whole (`*_target` / `*_source`: the two
+    meshes of each pair); per-vertex results for a fixed, seeded sample of DUMP_ROWS vertex positions, the same for
+    targets and sources, so that two builds given the same arguments can be compared output for output."""
+    import torch
+
+    def cat(fn):
+        return torch.cat([fn(o, o["spectral_weights"].shape[0]) for o in outs])
+
+    n_vert = outs[0]["final_idx"].shape[0] // outs[0]["spectral_weights"].shape[0]   # every mesh has n_vert vertices
+    tgt_vecs = cat(lambda o, p: o["eig_vecs"][:p * n_vert, :n_eig])
+    rows = np.sort(np.random.RandomState(0).choice(tgt_vecs.shape[0], min(DUMP_ROWS, tgt_vecs.shape[0]), replace=False))
+    rows_d = torch.from_numpy(rows).to(tgt_vecs.device)
+    arrays = {"eig_vals_target": cat(lambda o, p: o["eig_vals"][:p, :n_eig]),
+              "eig_vals_source": cat(lambda o, p: o["eig_vals"][p:, :n_eig]),
+              "Q": cat(lambda o, p: o["Q"]),
+              "spectral_weights": cat(lambda o, p: o["spectral_weights"]),
+              "sample_vertex_rows": torch.from_numpy(rows),
+              "eig_vecs_target": tgt_vecs[rows_d],
+              "eig_vecs_source": cat(lambda o, p: o["eig_vecs"][p * n_vert:, :n_eig])[rows_d]}
+    for key in ("final_idx", "weighted_avg_transformed_points", "nearest_neighbor_transformed_points"):
+        arrays[key] = cat(lambda o, p: o[key])[rows_d]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy().astype(np.float64))
 
 
 def run_reference(a):
@@ -215,18 +249,26 @@ def run_ours(a):
         d2h[0] = S * sum(v.nbytes for v in sb.fetch(out, slot=None).values())
         return out["eigs_info"]
 
-    def run_steps(steps, e2e):
+    def run_steps(steps, e2e, keep_outputs=False):
         """`steps` steps of the hot path over this rank's pairs.  A step is either ONE batch of all P pairs (S = 1) with
         up to D steps in flight (SpectralBatch.run_pipelined: kernels keep their full size, the tail of a step hides under
-        the filter of the next), or S sub-batches of P / S pairs run concurrently (SpectralBatch.run_concurrent)."""
+        the filter of the next), or S sub-batches of P / S pairs run concurrently (SpectralBatch.run_concurrent).
+        keep_outputs: the last step's results (device tensors) stay referenced in last["outputs"] for --dump-outputs."""
         js, consume = (jobs_e2e if e2e else jobs), (fetch_results if e2e else keep_info)
         if S == 1:
+            if keep_outputs:
+                def consume(out, k, base=consume):
+                    if k == steps - 1:
+                        last["outputs"] = [{key: out[key] for key in DUMP_KEYS}]
+                    return base(out, k)
             infos = sb.run_pipelined([js[0]] * steps, depth=D, consume=consume)
             last["infos"] = infos[-1:]
         else:
             for _ in range(steps):
                 outs = sb.run_concurrent(js)
                 last["infos"] = [consume(o, k) for k, o in enumerate(outs)]
+            if keep_outputs:
+                last["outputs"] = [{key: o[key] for key in DUMP_KEYS} for o in outs]
 
     def timed(fn, steps):
         barrier()
@@ -241,9 +283,14 @@ def run_ours(a):
     sampler = ClockSampler(local) if rank == 0 else None
     lib.focusr_profile_reset()
     l0 = _lib.launch_count()
-    ms = timed(lambda k: run_steps(k, False), a.steps)
+    ms = timed(lambda k: run_steps(k, False, keep_outputs=bool(a.dump_outputs)), a.steps)
     launches = _lib.launch_count() - l0
     max_residual, fp32_steps, filter_steps = certify(last["infos"])
+    if a.dump_outputs:
+        outputs = last.pop("outputs")
+        if rank == 0:
+            dump_outputs(outputs, sb.n, a.dump_outputs)
+        del outputs
     max_residual = fdist.all_reduce_max(max_residual)
     # With several streams in flight (steps, sub-batches, the smoothing side stream) launches interleave and a kernel's
     # duration is not defined; the per-kernel numbers (roofline) come from the same K steps run again right away, still
@@ -705,7 +752,13 @@ def main():
     ap.add_argument("--no-rowpart", action="store_true", help="skip the 1M-vertex solve reported under secondary_metrics")
     ap.add_argument("--no-dense", action="store_true", help="skip the KNN / k = 65 FP64 evidence reported under secondary_metrics")
     ap.add_argument("--no-nonsym", action="store_true", help="skip the non-symmetric batch reported under secondary_metrics")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (rank 0's pairs) to DIR/<name>.npy in float64")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's results; the reference arm has none to write")
     return run_reference(a) if a.impl == "reference" else run_ours(a)
 
 
