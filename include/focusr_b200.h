@@ -192,7 +192,7 @@ int focusr_eigs_smallest_dist(const int* row_ptr, const int* cols_local, const d
  * stream around every filter application since the last reset): out4_host = {milliseconds,
  * launches, algorithmic bytes (12 nnz + 20 N + 24 b N per launch), 0}.  bench.py's roofline line.
  * focusr_profile_get counts the fp64 steps (k_spmm); focusr_profile_get_kind(kind, ...) the steps of one kind:
- * 0 = fp64, 1 = fp32 (k_spmm_f32: 8 nnz + 12 N + 12 b N per launch), 2 = fp32 correction form (k_spmm_corr:
+ * 0 = fp64, 1 = fp32 (k_filter_sell mode 0: 8 nnz + 12 N + 12 b N per launch), 2 = fp32 correction form (mode 3:
  * 8 nnz + 12 N + 16 b N per launch); reset clears all three.  kind 3 = the persistent filter kernels of the last
  * row-partitioned solve of this process: {nanoseconds CTA 0 spent at the in-kernel barriers, nanoseconds it spent
  * working, steps, 0}.  kind 4 = the pruned KNN: {(query, reference) distance evaluations since the last reset, 0, 0,

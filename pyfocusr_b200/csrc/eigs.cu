@@ -558,7 +558,7 @@ static thread_local PinnedPool g_pin_small, g_pin_tables, g_pin_cut;
 // Live profile of the dominant kernel (the Chebyshev SpMM step): CUDA events bracket every
 // filter() on the launching stream; the elapsed time is collected at the next synchronisation the
 // driver performs anyway.  bench.py turns {ms, launches, algorithmic bytes} into the roofline line.
-// fp32 filter passes (chfsi_driver.hpp, k_spmm_f32): a pass may run in fp32 if it is meant to leave every residual
+// fp32 filter passes (chfsi_driver.hpp, k_filter_sell in sell.cu): a pass may run in fp32 if it is meant to leave every residual
 // above this value.  The fp32 floor measured on 15k-vertex meshes is ~5e-7 (a pass aimed lower stalls there).
 constexpr double LOWP_FLOOR = 1.4e-6;
 // A sized plain-fp32 pass aims here (lands at ~0.7 of its aim): low enough for the fp32 correction form to reach 1e-10
@@ -608,7 +608,7 @@ struct FilterProfile {
     pending = false;
   }
 };
-static FilterTotals g_totals[3];  // fp64 steps (k_spmm<b,.,0>), fp32 steps (k_spmm_f32), fp32 correction steps (k_spmm_corr)
+static FilterTotals g_totals[3];  // fp64 steps (k_spmm<b,.,0>), fp32 steps (k_filter_sell modes 0-2), fp32 correction steps (modes 3-4)
 static thread_local FilterProfile g_filter_profile(&g_totals[0]);
 static thread_local FilterProfile g_filter_profile_lowp(&g_totals[1]);
 static thread_local FilterProfile g_filter_profile_corr(&g_totals[2]);

@@ -43,8 +43,7 @@ struct FilterTuning {
 
 // One Chebyshev filter step on the SELL copy.  mode: 0 plain fp32 step (y, x_prev, out fp32), 1 first step of a pass (y
 // fp64 -> out fp32, y_copy = fp32 copy of y), 2 last step (out fp64), 3 correction step (z, z_prev, r -> z_next; per-column
-// float tables), 4 last correction step (x += z_next in fp64).  Same arithmetic, operand order and results as
-// k_spmm_f32 / k_spmm_corr.
+// float tables), 4 last correction step (x += z_next in fp64).
 int launch_filter_sell(int mode, int b, const SellF32& m, const int* mesh_off, int n_meshes, int max_mesh_rows,
                        const void* y, const float* x_prev, const float* r, void* out, float* y_copy,
                        const void* alpha, const void* gamma, const double* center, int step, int n_steps, bool has_prev,

@@ -210,7 +210,7 @@ struct HostBackend {
     std::memcpy(th, theta.data(), theta.size() * sizeof(double));
     std::memcpy(rs, res.data(), res.size() * sizeof(double));
   }
-  // fp32 pass as k_spmm_f32 runs it: blocks, matrix entries and table values rounded to float, float arithmetic
+  // fp32 pass as k_filter_sell (modes 0-2) runs it: blocks, matrix entries and table values rounded to float, float arithmetic
   void filter_lowp(int deg_m, const double* alpha, const double* gamma, const double* center) {
     std::vector<float> p(X.size()), y(X.size()), n(X.size()), acc(B);
     for (size_t t = 0; t < X.size(); ++t) y[t] = (float)X[t];
@@ -239,7 +239,7 @@ struct HostBackend {
     }
     for (size_t t = 0; t < X.size(); ++t) X[t] = (double)y[t];
   }
-  // fp32 correction pass as k_spmm_corr runs it: X += z_deg, z_{k+1} = alpha_kj ((L - c) z_k + r_j) - gamma_kj z_{k-1}, z_0 = 0;
+  // fp32 correction pass as k_filter_sell (modes 3-4) runs it: X += z_deg, z_{k+1} = alpha_kj ((L - c) z_k + r_j) - gamma_kj z_{k-1}, z_0 = 0;
   // z, r, matrix entries and tables rounded to float, float arithmetic; tables are [mesh][step][column]
   void filter_correction(int deg_m, const double* a_m, const double* beta_m) {
     // the per-column tables, as k_corr_tables builds them on the GPU

@@ -224,7 +224,9 @@ def test_eigs_mixed_precision_passes(torch, shipped_meshes, synth, block):
     """By default the filter passes iterate in fp32 (k_filter_sell on the sliced-ELL fp32 copy of the matrix: plain fp32
     blocks, then the correction form driven by the fp64 residual; float4 slices, 2 or 4 threads per row);
     options.mixed_precision = 0 keeps fp64 throughout.  Both meet the fp64 tolerance and the oracle; the fp32 passes cost
-    no extra filter degree.  Every cache-policy / occupancy variant of the kernels gives bit-identical eigenvectors."""
+    no extra filter degree.  The eigenvectors do not change with the filter options.  This batch is small enough that
+    the filter steps run one pass per CTA, a form that ignores filter_policy, so the loop below varies only the prefetch
+    and the resident-CTA build; test_gpu_kernels.py checks every cache policy on the 256-row form step by step."""
     from pyfocusr_b200._device import DeviceGraph
 
     ms = [shipped_meshes["target_mesh"], synth["ell20a"], synth["ell39"]]

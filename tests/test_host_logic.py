@@ -192,7 +192,7 @@ def test_driver_symmetric_batch(hostsim, shipped_meshes):
 
 
 def test_driver_mixed_precision_passes(hostsim, shipped_meshes):
-    """Filter passes in fp32 (the test double rounds as k_spmm_f32 / k_spmm_corr do): a pass that lands above the fp32
+    """Filter passes in fp32 (the test double rounds as the k_filter_sell steps do): a pass that lands above the fp32
     floor runs on fp32 blocks, the pass that reaches the tolerance runs in fp32 correction form (z = p(L)x - x driven by
     the fp64 residual).  Rayleigh-Ritz and residuals stay fp64, so tolerance and parity hold, at no extra degree."""
     ms = [shipped_meshes["target_mesh"], fmesh.perturbed_ellipsoid(20, 3)]
