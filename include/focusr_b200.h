@@ -196,7 +196,8 @@ int focusr_eigs_smallest_dist(const int* row_ptr, const int* cols_local, const d
  * 8 nnz + 12 N + 16 b N per launch); reset clears all three.  kind 3 = the persistent filter kernels of the last
  * row-partitioned solve of this process: {nanoseconds CTA 0 spent at the in-kernel barriers, nanoseconds it spent
  * working, steps, 0}.  kind 4 = the pruned KNN: {(query, reference) distance evaluations since the last reset, 0, 0,
- * 0} (synchronises the device). */
+ * 0} (synchronises the device).  kind 5 = the ICP closest-point search: {(landmark, triangle) evaluations since the last
+ * reset, 0, 0, 0}, counted only by a build with -DFB_ICP_COUNT (0 otherwise; synchronises the device). */
 void focusr_profile_reset(void);
 void focusr_profile_get(double* out4_host);
 void focusr_profile_get_kind(int kind, double* out4_host);
@@ -359,6 +360,10 @@ int focusr_curvatures(const double* points, const int* tris, int n_points, int n
  * vectors (vtkMatrix4x4 layout); transformed_out: device [n_source_points][3] = matrix * source (the
  * `apply_transform` of vtk_functions.py:32-37); both nullable.  Target triangle ids must be in range
  * (checked by focusr_laplacian_build on the same mesh).  Does not synchronise.
+ * The closest point of a landmark is the exact one of a scan over all target triangles (the lowest triangle index
+ * wins a tie); the search visits Morton-ordered tiles of 32 triangles and skips those whose padded box is strictly
+ * farther than the best distance known, which changes no result.  focusr_icp is the one-pair case of
+ * focusr_icp_batch: a pair's result does not depend on the batch it is in.
  * ------------------------------------------------------------------------------------------- */
 size_t focusr_icp_workspace_bytes(int n_source_points, int n_target_tris);
 int focusr_icp(const double* target_points, int n_target_points, const int* target_tris,
@@ -366,6 +371,26 @@ int focusr_icp(const double* target_points, int n_target_points, const int* targ
                int max_iterations, int similarity, int start_by_matching_centroids,
                double* matrix_out, double* transformed_out, void* workspace, size_t workspace_bytes,
                focusr_stream_t stream);
+
+/* K10, batched: n_pairs registrations in one set of launches per iteration, on the batch layout (`points`
+ * [n_points][3], `tris` with global vertex ids, mesh m = rows mesh_off[m] .. mesh_off[m+1] and triangles
+ * tri_off[m] .. tri_off[m+1], i.e. `tris` grouped by mesh).  Pair p moves mesh moving_mesh[p] onto the surface of
+ * mesh fixed_mesh[p], with the arguments and results of focusr_icp for that pair alone (bit-identical).  The
+ * `_host` arrays are host copies of the device arrays of the same name (launch sizing and argument checks).
+ * A fixed mesh without triangles, an empty mesh, or a mesh that moves in more than one pair is an argument error.
+ * matrices: device [n_pairs][16] (nullable); moved_points: device [n_points][3] (nullable, must not alias
+ * `points`): the rows of every moving mesh = its matrix * its points, all other rows copied unchanged.
+ * Does not synchronise.  The workspace size is 0 for an invalid description. */
+size_t focusr_icp_batch_workspace_bytes(const int* mesh_off_host, const int* tri_off_host, int n_meshes,
+                                        const int* fixed_mesh_host, const int* moving_mesh_host, int n_pairs,
+                                        int max_landmarks);
+int focusr_icp_batch(const double* points, int n_points, const int* tris, const int* mesh_off,
+                     const int* mesh_off_host, const int* tri_off, const int* tri_off_host, int n_meshes,
+                     const int* fixed_mesh, const int* moving_mesh, const int* fixed_mesh_host,
+                     const int* moving_mesh_host, int n_pairs, int max_landmarks, int max_iterations,
+                     int similarity, int start_by_matching_centroids, double* matrices,
+                     double* moved_points, void* workspace, size_t workspace_bytes,
+                     focusr_stream_t stream);
 
 #ifdef __cplusplus
 }

@@ -343,6 +343,61 @@ def icp(target_points, target_tris, source_points, max_iterations=100, max_landm
     return mat.cpu().numpy().reshape(4, 4), moved
 
 
+def icp_landmarks(n_points, max_landmarks):
+    """The landmark rule of ``focusr_icp`` / ``focusr_icp_batch`` (vtkIterativeClosestPointTransform::InternalUpdate):
+    every ``step``-th point of a moving mesh of ``n_points`` is a landmark.  Returns ``(step, count)``."""
+    n, ml = int(n_points), int(max_landmarks)
+    step = n // ml if n > ml else 1
+    return step, n // step
+
+
+def icp_batch_device(points, tris, mesh_off_host, tri_off_host, fixed_mesh, moving_mesh, max_iterations=100,
+                     max_landmarks=1000, similarity=False, start_by_matching_centroids=True):
+    """``focusr_icp_batch`` on device tensors; returns ``(matrices (P, 4, 4) float64, moved (N, 3) float64)``, both on
+    the device, without synchronising.  ``points`` is not modified."""
+    torch = _torch()
+    lib = _lib.load()
+    dev = points.device
+    off = np.ascontiguousarray(mesh_off_host, dtype=np.int32)
+    toff = np.ascontiguousarray(tri_off_host, dtype=np.int32)
+    fm = np.ascontiguousarray(fixed_mesh, dtype=np.int32).reshape(-1)
+    mm = np.ascontiguousarray(moving_mesh, dtype=np.int32).reshape(-1)
+    m, P, n = off.size - 1, int(fm.size), int(points.shape[0])
+    if toff.size != off.size or mm.size != P:
+        raise ValueError("icp_batch: tri_off_host needs n_meshes + 1 entries and every pair a fixed and a moving mesh")
+    nbytes = int(lib.focusr_icp_batch_workspace_bytes(_lib.ptr(off), _lib.ptr(toff), m, _lib.ptr(fm), _lib.ptr(mm), P,
+                                                      int(max_landmarks)))
+    ws = torch.empty(max(nbytes, 1), dtype=torch.uint8, device=dev)
+    off_d, toff_d, fm_d, mm_d = (torch.from_numpy(a).to(dev, non_blocking=True) for a in (off, toff, fm, mm))
+    mats = torch.empty((P, 4, 4), dtype=torch.float64, device=dev)
+    moved = torch.empty_like(points)
+    _lib.call("focusr_icp_batch", _lib.ptr(points), n, _lib.ptr(tris), _lib.ptr(off_d), _lib.ptr(off), _lib.ptr(toff_d),
+              _lib.ptr(toff), m, _lib.ptr(fm_d), _lib.ptr(mm_d), _lib.ptr(fm), _lib.ptr(mm), P, int(max_landmarks),
+              int(max_iterations), int(bool(similarity)), int(bool(start_by_matching_centroids)), _lib.ptr(mats),
+              _lib.ptr(moved), _lib.ptr(ws), nbytes, _lib.stream_ptr())
+    return mats, moved
+
+
+def icp_batch(points, tris, mesh_off_host, tri_off_host, fixed_mesh, moving_mesh, max_iterations=100,
+              max_landmarks=1000, similarity=False, start_by_matching_centroids=True):
+    """vtkIterativeClosestPointTransform for many pairs at once (``focusr_icp_batch``): pair p moves mesh
+    ``moving_mesh[p]`` onto the surface of mesh ``fixed_mesh[p]`` of the batch (``points`` (N, 3) float64, ``tris``
+    (F, 3) int32 with global vertex ids grouped by mesh, host or device; ``mesh_off_host`` / ``tri_off_host`` the
+    per-mesh row and triangle ranges).  Each pair's result is that of :func:`icp` on the pair alone.  Returns
+    ``(matrices (P, 4, 4) host numpy, moved points (N, 3) device tensor)``: the rows of meshes that do not move are
+    copied unchanged."""
+    torch = _torch()
+
+    def dev(a, dt):
+        t = a if isinstance(a, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(a))
+        return t.to(device="cuda", dtype=dt).contiguous()
+
+    mats, moved = icp_batch_device(dev(points, torch.float64), dev(tris, torch.int32), mesh_off_host, tri_off_host,
+                                   fixed_mesh, moving_mesh, max_iterations, max_landmarks, similarity,
+                                   start_by_matching_centroids)
+    return mats.cpu().numpy(), moved
+
+
 def curvatures(points, tris):
     """vtkCurvatures on the device (vtk_functions.py:40-74).  ``points`` (N, 3) f64, ``tris`` (F, 3) i32, host or
     device.  Returns a dict of device tensors ``gauss``, ``mean``, ``minimum``, ``maximum``, each (N,)."""

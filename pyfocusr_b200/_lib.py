@@ -72,6 +72,9 @@ SIGNATURES = {
     "focusr_curvatures": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "focusr_icp_workspace_bytes": (_sz, [_i, _i]),
     "focusr_icp": (_i, [_vp, _i, _vp, _i, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _sz, _vp]),
+    "focusr_icp_batch_workspace_bytes": (_sz, [_vp, _vp, _i, _vp, _vp, _i, _i]),
+    "focusr_icp_batch": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp,
+                              _sz, _vp]),
     "focusr_cpd_workspace_bytes": (_sz, [_i, _i, _i, _i]),
     "focusr_cpd_affine": (_i, [_vp, _i, _vp, _i, _i, _i, _d, _d, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "focusr_cpd_deformable": (_i, [_vp, _i, _vp, _i, _i, _i, _d, _d, _d, _d, _i, _vp, _vp, _vp, _vp, _sz, _vp]),

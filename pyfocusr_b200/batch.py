@@ -30,7 +30,8 @@ class SpectralBatch:
                  block_size=0, seed=0, registration="identity", n_coords_spectral_registration=5000,
                  rigid_before_non_rigid_reg=True, rigid_reg_max_iterations=100, rigid_tolerance=1e-8,
                  non_rigid_max_iterations=1000, non_rigid_tolerance=1e-8, non_rigid_alpha=0.5, non_rigid_beta=3.0,
-                 non_rigid_n_eigens=100, cpd_streams=8):
+                 non_rigid_n_eigens=100, cpd_streams=8, icp_register_first=False, icp_registration_mode="rigid",
+                 icp_reg_target_to_source=False):
         self.ns = int(n_spectral_features)
         self.n = int(n_spectral_features + n_extra_spectral)
         self.n_samples = int(n_coords_spectral_ordering)
@@ -53,6 +54,14 @@ class SpectralBatch:
                                non_rigid_max_iterations=non_rigid_max_iterations, non_rigid_tolerance=non_rigid_tolerance,
                                non_rigid_alpha=non_rigid_alpha, non_rigid_beta=non_rigid_beta,
                                non_rigid_n_eigens=non_rigid_n_eigens)
+        # focusr.py:106-131 with Focusr's keyword names: rigid ("rigid") or similarity ("similarity") ICP, 100 iterations x
+        # 1000 landmarks, of every pair's source onto its target (or the target onto its source), before the Laplacian
+        # build; off by default
+        if icp_registration_mode not in ("rigid", "similarity"):
+            raise TypeError("icp_registration_mode must be 'rigid' or 'similarity', got %r" % (icp_registration_mode,))
+        self.icp_register_first = bool(icp_register_first)
+        self.icp_registration_mode = icp_registration_mode
+        self.icp_reg_target_to_source = bool(icp_reg_target_to_source)
         self._tls = threading.local()
         self._pool = None
         self.eigs_options = None  # _lib.EigsOptions or dict: per-call options of the eigensolver (A/B measurements)
@@ -82,10 +91,16 @@ class SpectralBatch:
 
     # ------------------------------------------------------------------------------------------
     def run(self, points, tris, mesh_off_host, n_pairs, idx_t=None, idx_s=None, record_events=False,
-            keep_presort=False):
+            keep_presort=False, tri_off_host=None):
         """points: torch tensor [n_points_total, 3] float64 (host pinned or device), meshes in the
         order targets then sources; tris: int32 [n_tris_total, 3] with GLOBAL vertex ids;
-        mesh_off_host: int32 [2P+1].  Returns a dict of device tensors + host metadata."""
+        mesh_off_host: int32 [2P+1].  Returns a dict of device tensors + host metadata.
+
+        With ``icp_register_first`` every pair's source is moved onto its target (or the target onto its source) in a
+        new device tensor before anything else; ``points`` is never modified and ``icp_matrices`` holds the (P, 4, 4)
+        matrices.  ICP needs each mesh's triangle range: ``tri_off_host`` int [2P+1], or else it is derived from
+        ``tris``, which must then be grouped by mesh in mesh order as ``pack_meshes`` makes them (``ValueError``
+        otherwise; for device ``tris`` the check reads one small result back to the host)."""
         torch = _lib.require_cuda()
         P = int(n_pairs)
         ev = []
@@ -97,6 +112,10 @@ class SpectralBatch:
                 ev.append((name, e))
 
         mark("start")
+        icp_mats = None
+        if self.icp_register_first:
+            points, tris, icp_mats = self._icp(points, tris, mesh_off_host, P, tri_off_host)
+            mark("icp")
         g = DeviceGraph.from_device(points, tris, mesh_off_host)
         mark("laplacian")
         n, ns = self.n, self.ns
@@ -189,7 +208,44 @@ class SpectralBatch:
                     source_projected_on_target=src_proj[nt_total:], final_idx=idx1[:, 0], knn3_idx=idx3,
                     knn3_dist=dist3, weighted_avg_transformed_points=weighted,
                     nearest_neighbor_transformed_points=nearest, idx_t=idx_t, idx_s=idx_s, costs=costs,
-                    eig_vecs_presort=presort, cpd_idx=cpd_idx, coords_b4_reg=coords_b4_reg)
+                    eig_vecs_presort=presort, cpd_idx=cpd_idx, coords_b4_reg=coords_b4_reg, icp_matrices=icp_mats)
+
+    def _icp(self, points, tris, mesh_off_host, P, tri_off_host):
+        """focusr.py:110-131 for every pair at once (``focusr_icp_batch``): returns the device points with each pair's
+        moving mesh registered onto its fixed one (a new tensor), the device triangles and the (P, 4, 4) matrices."""
+        torch = _lib.require_cuda()
+        off = np.ascontiguousarray(mesh_off_host, dtype=np.int32)
+        if tri_off_host is None:
+            tri_off_host = self.tri_offsets(tris, off)
+        dev = torch.device("cuda", torch.cuda.current_device())
+        pts = points.to(dev, non_blocking=True).contiguous()
+        tr = tris.to(dev, non_blocking=True).contiguous()
+        targets, sources = np.arange(P, dtype=np.int32), np.arange(P, 2 * P, dtype=np.int32)
+        fixed, moving = (sources, targets) if self.icp_reg_target_to_source else (targets, sources)
+        mats, moved = _device.icp_batch_device(pts, tr, off, tri_off_host, fixed, moving, max_iterations=100,
+                                               max_landmarks=1000, similarity=self.icp_registration_mode == "similarity")
+        return moved, tr, mats
+
+    @staticmethod
+    def tri_offsets(tris, mesh_off_host):
+        """Per-mesh triangle ranges int32 [M+1] of ``tris`` (torch int [F, 3], global vertex ids, host or device), which
+        must be grouped by mesh in mesh order (every triangle's vertices in one mesh, meshes non-decreasing), as
+        ``pack_meshes`` makes them; ``ValueError`` otherwise.  Device ``tris`` cost one small read back to the host."""
+        import torch
+
+        off = np.ascontiguousarray(mesh_off_host, dtype=np.int64)
+        m = off.size - 1
+        t = torch.as_tensor(tris).reshape(-1, 3).to(torch.int64)
+        mesh = torch.bucketize(t, torch.from_numpy(off[1:-1].copy()).to(t.device), right=True)  # mesh of every vertex id
+        m0 = mesh[:, 0]
+        ok = (mesh == m0[:, None]).all() & (t >= int(off[0])).all() & (t < int(off[-1])).all() & (m0[1:] >= m0[:-1]).all()
+        res = torch.cat([ok.reshape(1).to(torch.int64), torch.bincount(m0, minlength=m)[:m]]).cpu().numpy()
+        if not res[0]:
+            raise ValueError("tris must be grouped by mesh in mesh order (as pack_meshes makes them) to derive the "
+                             "per-mesh triangle ranges; pass tri_off_host otherwise")
+        tri_off = np.zeros(m + 1, dtype=np.int32)
+        tri_off[1:] = np.cumsum(res[1:])
+        return tri_off
 
     # ------------------------------------------------------------------------------------------
     def run_concurrent(self, sub_batches, **kw):
@@ -400,4 +456,7 @@ class SpectralBatch:
     def run_meshes(self, targets, sources, **kw):
         """Convenience: lists of PolyData-like meshes (``.points``, ``.tris``)."""
         pts, tris, off, n_pairs = self.pack_meshes(targets, sources)
+        tri_off = np.zeros(len(targets) + len(sources) + 1, dtype=np.int32)
+        tri_off[1:] = np.cumsum([m.tris.shape[0] for m in list(targets) + list(sources)])
+        kw.setdefault("tri_off_host", tri_off)
         return self.run(pts, tris, off, n_pairs, **kw)

@@ -23,6 +23,7 @@
 namespace fb {
 
 unsigned long long pk_evals_read_and_maybe_reset(bool reset);  // knn_pruned.cu
+unsigned long long icp_evals_read_and_maybe_reset(bool reset);  // icp.cu
 
 constexpr int GRAM_ROWS = 1024;  // rows per CTA (8 warps x 128 rows)
 constexpr int GRAM_THREADS = 256;
@@ -1344,6 +1345,7 @@ extern "C" {
 
 void focusr_profile_reset(void) {
   pk_evals_read_and_maybe_reset(true);
+  icp_evals_read_and_maybe_reset(true);
   g_filter_profile.collect();
   g_filter_profile_lowp.collect();
   g_filter_profile_corr.collect();
@@ -1357,6 +1359,13 @@ void focusr_profile_get_kind(int kind, double* out4_host) {
   if (kind == 4) {  // pruned KNN: (query, reference) distance evaluations since the last reset (synchronises the device)
     cudaDeviceSynchronize();
     out4_host[0] = (double)pk_evals_read_and_maybe_reset(false);
+    out4_host[1] = out4_host[2] = out4_host[3] = 0.0;
+    return;
+  }
+  if (kind == 5) {  // ICP closest-point search: (landmark, triangle) evaluations since the last reset, counted only in
+                    // builds with -DFB_ICP_COUNT (synchronises the device)
+    cudaDeviceSynchronize();
+    out4_host[0] = (double)icp_evals_read_and_maybe_reset(false);
     out4_host[1] = out4_host[2] = out4_host[3] = 0.0;
     return;
   }

@@ -13,6 +13,7 @@
 
 #include "common.cuh"
 #include "knn.cuh"
+#include "morton.cuh"
 #include "rowops.h"
 
 namespace fb {
@@ -33,30 +34,6 @@ constexpr int PK_TR = FB_PK_TR;  // references per tile (A/B builds: tools/knn_a
 constexpr int PK_TQ = FB_PK_TQ;  // queries per CTA
 constexpr int PK_SORT_MAX = 16384;
 constexpr int PK_MAX_DIM = 32;
-
-__device__ __forceinline__ unsigned spread10(unsigned v) {  // 10 bits -> every third bit
-  v &= 0x3ffu;
-  v = (v | (v << 16)) & 0x030000ffu;
-  v = (v | (v << 8)) & 0x0300f00fu;
-  v = (v | (v << 4)) & 0x030c30c3u;
-  v = (v | (v << 2)) & 0x09249249u;
-  return v;
-}
-
-__device__ __forceinline__ unsigned morton3(const double* p, int dim, const double* lo, const double* inv) {
-  unsigned key = 0;
-#pragma unroll
-  for (int c = 0; c < 3; ++c) {
-    unsigned q = 0;
-    if (c < dim) {
-      double t = (p[c] - lo[c]) * inv[c];
-      t = fmin(fmax(t, 0.0), 1023.0);
-      q = (unsigned)t;
-    }
-    key |= spread10(q) << c;
-  }
-  return key;
-}
 
 // bounding box of refs U queries of each segment over the first min(dim,3) coordinates
 __global__ void __launch_bounds__(256)
