@@ -352,6 +352,36 @@ int focusr_curvatures(const double* points, const int* tris, int n_points, int n
                       size_t workspace_bytes, focusr_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * K12  Node features of a batch (csrc/features.cu), for every mesh m = rows mesh_point_off[m] .. [m+1].  Neither call
+ * allocates, synchronises or reads anything back; one CTA per (mesh, column) / per mesh, no floating-point atomics, so
+ * a mesh's results do not depend on the batch it is in.  Results equal numpy's bit for bit: mean and std follow
+ * numpy's pairwise summation tree, products are rounded before they are added, min / max propagate NaN.
+ *
+ * focusr_node_features: Graph.norm_node_features (graph.py:121-142) for every (mesh, column) of `raw` [n_points]
+ * [n_features] (curvature columns, then mesh scalars): if norm_std, f = (f - mean(f)) / std(f), then, if has_cap,
+ * f[f > cap] = cap and f[f < -cap] = -cap (the reference caps for any cap that is not False, 0 included); if norm_0_1,
+ * f = (f - min f) / ptp f.  features_out [n_points][n_features].  edge_points (nullable) [n_points][3 + n_features] =
+ * xyz followed by f * mean_pts_scale_range, mean_pts_scale_range = ((ptp x + ptp y) + ptp z) / 3 of the mesh's
+ * `points` [n_points][3] (graph.py:166-175): the `points` focusr_laplacian_build takes when features are in the edge
+ * weights.  A feature with zero spread gives NaN, as in numpy; the Laplacian build counts the non-finite weights.
+ * n_features <= 61.
+ *
+ * focusr_feature_coords: the extended correspondence coordinates of focusr.py:218-295, out [n_points]
+ * [ns + n_features + 3 * include_points]: the `spectral` [n_points][ns] columns; then, per smoothed feature g
+ * (`smoothed_features` [n_points][n_features], nullable when n_features = 0), ptp(spectral of the mesh) *
+ * ((g - min g) / max(g - min g)); then, if include_points, (p - min p) / mean_pts_scale_range (norm_physical_and_spectral)
+ * or raw xyz after every earlier column was multiplied by mean_pts_scale_range (not norm_physical_and_spectral).
+ * ------------------------------------------------------------------------------------------- */
+size_t focusr_node_features_workspace_bytes(int n_points, int n_meshes, int n_features);
+int focusr_node_features(const double* raw, const double* points, int n_points, const int* mesh_point_off,
+                         int n_meshes, int n_features, int norm_std, int has_cap, double cap, int norm_0_1,
+                         double* features_out, double* edge_points, void* workspace, size_t workspace_bytes,
+                         focusr_stream_t stream);
+int focusr_feature_coords(const double* spectral, int ns, const double* smoothed_features, int n_features,
+                          const double* points, int n_points, const int* mesh_point_off, int n_meshes,
+                          int include_points, int norm_physical_and_spectral, double* out, focusr_stream_t stream);
+
+/* ---------------------------------------------------------------------------------------------
  * K10  ICP pre-alignment (focusr.py:106-131 -> vtk_functions.py:12-37: vtkIterativeClosestPointTransform
  * with a rigid-body (similarity = 0) or similarity landmark transform, closest points ON the target
  * surface, StartByMatchingCentroids, exactly max_iterations landmark fits; landmarks = every

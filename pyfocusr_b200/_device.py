@@ -45,14 +45,15 @@ class DeviceGraph:
         self._init_from_host(torch.from_numpy(pts), torch.from_numpy(np.ascontiguousarray(tris)), edge_pts)
 
     @classmethod
-    def from_device(cls, points, tris, mesh_off_host):
-        """Build from tensors that are already resident in HBM (``tris`` hold global ids)."""
+    def from_device(cls, points, tris, mesh_off_host, edge_points=None):
+        """Build from tensors that are already resident in HBM (``tris`` hold global ids).  ``edge_points`` (optional,
+        [n_points][3+f]): the coordinates the edge weights are measured in (``node_features``); ``points`` stays xyz."""
         self = cls.__new__(cls)
         self.mesh_off_host = np.ascontiguousarray(mesh_off_host, dtype=np.int32)
         self.n_meshes = self.mesh_off_host.size - 1
         self.n_points = int(self.mesh_off_host[-1])
         self.max_mesh_points = int(np.max(np.diff(self.mesh_off_host)))
-        self._init_from_host(points, tris)
+        self._init_from_host(points, tris, edge_points)
         return self
 
     def _init_from_host(self, points, tris, edge_points=None):
@@ -414,6 +415,42 @@ def curvatures(points, tris):
     _lib.call("focusr_curvatures", _lib.ptr(pts), _lib.ptr(tr), n, f, _lib.ptr(out[0]), _lib.ptr(out[1]), _lib.ptr(out[2]),
               _lib.ptr(out[3]), _lib.ptr(ws), nbytes, _lib.stream_ptr())
     return dict(gauss=out[0], mean=out[1], minimum=out[2], maximum=out[3])
+
+
+def node_features(raw, points, mesh_off, norm_std=True, cap=3, norm_0_1=True, want_edge_points=False):
+    """Graph.norm_node_features (graph.py:121-142) for every (mesh, column) of a batch (``focusr_node_features``).
+    ``raw`` device [n_points][f] float64, ``points`` device [n_points][3], ``mesh_off`` device int32 [n_meshes + 1].
+    ``cap``: any value but ``False`` caps at +-cap, as the reference does.  Returns ``(features [n_points][f],
+    edge_points [n_points][3 + f] or None)``: xyz followed by the features times each mesh's mean xyz range
+    (graph.py:166-175).  Does not synchronise."""
+    torch = _torch()
+    lib = _lib.load()
+    n, f, m = int(raw.shape[0]), int(raw.shape[1]), int(mesh_off.shape[0]) - 1
+    out = torch.empty((n, f), dtype=torch.float64, device=raw.device)
+    ep = torch.empty((n, 3 + f), dtype=torch.float64, device=raw.device) if want_edge_points else None
+    ws_bytes = int(lib.focusr_node_features_workspace_bytes(n, m, f))
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=raw.device)
+    has_cap = cap is not False
+    _lib.call("focusr_node_features", _lib.ptr(raw), _lib.ptr(points), n, _lib.ptr(mesh_off), m, f, int(norm_std is True),
+              int(has_cap), float(cap) if has_cap else 0.0, int(norm_0_1 is True), _lib.ptr(out), _lib.ptr(ep), _lib.ptr(ws),
+              ws_bytes, _lib.stream_ptr())
+    return out, ep
+
+
+def feature_coords(spectral, smoothed, points, mesh_off, include_points=False, norm_physical_and_spectral=True):
+    """The extended correspondence coordinates of focusr.py:218-295 for every mesh of a batch (``focusr_feature_coords``):
+    ``spectral`` device [n_points][ns], then the smoothed features ``smoothed`` [n_points][f] (or None) rescaled to each
+    mesh's spectral range, then, with ``include_points``, the normed (or raw) xyz of ``points``.  Returns a new device
+    tensor [n_points][ns + f + 3 * include_points]."""
+    torch = _torch()
+    n, ns = int(spectral.shape[0]), int(spectral.shape[1])
+    f = 0 if smoothed is None else int(smoothed.shape[1])
+    m = int(mesh_off.shape[0]) - 1
+    out = torch.empty((n, ns + f + (3 if include_points else 0)), dtype=torch.float64, device=spectral.device)
+    _lib.call("focusr_feature_coords", _lib.ptr(spectral), ns, _lib.ptr(smoothed), f, _lib.ptr(points), n,
+              _lib.ptr(mesh_off), m, int(bool(include_points)), int(bool(norm_physical_and_spectral)), _lib.ptr(out),
+              _lib.stream_ptr())
+    return out
 
 
 def eigsort_decide(graph, vals, n_found, t_mesh, s_mesh, costs, n_features, ns, target_as_reference=True, weighted=True):

@@ -70,6 +70,9 @@ SIGNATURES = {
     "focusr_weighted_positions": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _vp]),
     "focusr_curvature_workspace_bytes": (_sz, [_i, _i]),
     "focusr_curvatures": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "focusr_node_features_workspace_bytes": (_sz, [_i, _i, _i]),
+    "focusr_node_features": (_i, [_vp, _vp, _i, _vp, _i, _i, _i, _i, _d, _i, _vp, _vp, _vp, _sz, _vp]),
+    "focusr_feature_coords": (_i, [_vp, _i, _vp, _i, _vp, _i, _vp, _i, _i, _i, _vp, _vp]),
     "focusr_icp_workspace_bytes": (_sz, [_i, _i]),
     "focusr_icp": (_i, [_vp, _i, _vp, _i, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _sz, _vp]),
     "focusr_icp_batch_workspace_bytes": (_sz, [_vp, _vp, _i, _vp, _vp, _i, _i]),

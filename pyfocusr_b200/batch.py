@@ -6,7 +6,8 @@ pairs sharded across 1/2/4/8 B200").  It is the same sequence ``Focusr.__init__`
 in BASELINE.md section 3), but every kernel works on the block-diagonal graph of all 2P meshes, so
 one SpMM launch streams gigabytes instead of 1.3 MB and nothing visits the host between the upload
 of the vertices and the download of the correspondences except the eigensolver's convergence test
-(a few hundred Ritz values and residuals per outer iteration).
+(a few hundred Ritz values and residuals per outer iteration) and, with node features on, the one synchronise of
+``focusr_curvatures`` (its triangle-index check).
 
 Mesh order inside the batch graph: targets 0..P-1, then sources 0..P-1.
 """
@@ -22,6 +23,19 @@ from ._device import DeviceGraph
 
 __all__ = ["SpectralBatch"]
 
+# graph.py:11-15 (features_dictionary): the focusr_curvatures outputs each name contributes, in order
+CURVATURE_FEATURES = {"curvature": ("minimum", "maximum"), "min_curvature": ("minimum",), "max_curvature": ("maximum",)}
+MAX_KNN_DIM, MAX_CPD_DIM = 32, 16  # focusr_knn, focusr_cpd_*
+
+
+def mesh_point_scalars(mesh, name):
+    """graph.py:88-119: the point scalars called ``name`` of a mesh (PolyData or vtkPolyData) as float64."""
+    pd = mesh.GetPointData()
+    for idx in range(pd.GetNumberOfArrays()):
+        if pd.GetArray(idx).GetName() == name:
+            return np.array(np.asarray(pd.GetArray(idx)), dtype=np.float64)
+    raise Exception("NO SCALARS WITH SPECIFIED NAME: %s" % name)
+
 
 class SpectralBatch:
     def __init__(self, n_spectral_features=3, n_extra_spectral=3, n_coords_spectral_ordering=5000,
@@ -31,7 +45,10 @@ class SpectralBatch:
                  rigid_before_non_rigid_reg=True, rigid_reg_max_iterations=100, rigid_tolerance=1e-8,
                  non_rigid_max_iterations=1000, non_rigid_tolerance=1e-8, non_rigid_alpha=0.5, non_rigid_beta=3.0,
                  non_rigid_n_eigens=100, cpd_streams=8, icp_register_first=False, icp_registration_mode="rigid",
-                 icp_reg_target_to_source=False):
+                 icp_reg_target_to_source=False, list_features_to_calc=("curvature",), list_features_to_get_from_mesh=(),
+                 include_features_in_adj_matrix=False, use_features_as_coords=False, feature_smoothing_iterations=40,
+                 norm_node_features_std=True, norm_node_features_cap_std=3, norm_node_features_0_1=True,
+                 include_points_as_features=False, norm_physical_and_spectral=True):
         self.ns = int(n_spectral_features)
         self.n = int(n_spectral_features + n_extra_spectral)
         self.n_samples = int(n_coords_spectral_ordering)
@@ -62,6 +79,36 @@ class SpectralBatch:
         self.icp_register_first = bool(icp_register_first)
         self.icp_registration_mode = icp_registration_mode
         self.icp_reg_target_to_source = bool(icp_reg_target_to_source)
+        # graph.py:84-142,166-175 and focusr.py:218-295 with Focusr's keyword names and meanings: node features (curvature
+        # columns, then mesh point scalars), normalised per mesh, in the edge weights and / or smoothed and appended to the
+        # correspondence coordinates; xyz appended to the coordinates.  The features are computed only when one of the
+        # two flags that consume them is set (otherwise the reference discards them), so the default call does no extra
+        # work.
+        unknown = [f for f in list_features_to_calc if f not in CURVATURE_FEATURES]
+        if unknown:
+            raise ValueError("unknown feature(s) %s: list_features_to_calc takes %s" % (unknown, sorted(CURVATURE_FEATURES)))
+        self.list_features_to_calc = list(list_features_to_calc)
+        self.list_features_to_get_from_mesh = list(list_features_to_get_from_mesh)
+        self.curvature_columns = [c for f in self.list_features_to_calc for c in CURVATURE_FEATURES[f]]
+        self.n_node_features = len(self.curvature_columns) + len(self.list_features_to_get_from_mesh)
+        self.include_features_in_adj_matrix = include_features_in_adj_matrix is True
+        self.use_features_as_coords = use_features_as_coords is True
+        self.feature_smoothing_iterations = int(feature_smoothing_iterations)
+        self.norm_node_features_std = norm_node_features_std
+        self.norm_node_features_cap_std = norm_node_features_cap_std
+        self.norm_node_features_0_1 = norm_node_features_0_1
+        self.include_points_as_features = include_points_as_features is True
+        self.norm_physical_and_spectral = norm_physical_and_spectral is True
+        self.features_in_adjacency = self.n_node_features > 0 and self.include_features_in_adj_matrix
+        self.features_as_coords = self.n_node_features > 0 and self.use_features_as_coords
+        self.features_on = self.features_in_adjacency or self.features_as_coords
+        self.n_coords = self.ns + (self.n_node_features if self.features_as_coords else 0) + \
+            (3 if self.include_points_as_features else 0)
+        if self.n_coords > MAX_KNN_DIM:
+            raise ValueError("correspondence coordinates of %d columns: the KNN stages take at most %d" % (self.n_coords, MAX_KNN_DIM))
+        if self.registration == "b200" and self.n_coords > MAX_CPD_DIM:
+            raise ValueError("correspondence coordinates of %d columns: registration='b200' (CPD) takes at most %d" % (
+                self.n_coords, MAX_CPD_DIM))
         self._tls = threading.local()
         self._pool = None
         self.eigs_options = None  # _lib.EigsOptions or dict: per-call options of the eigensolver (A/B measurements)
@@ -91,7 +138,7 @@ class SpectralBatch:
 
     # ------------------------------------------------------------------------------------------
     def run(self, points, tris, mesh_off_host, n_pairs, idx_t=None, idx_s=None, record_events=False,
-            keep_presort=False, tri_off_host=None):
+            keep_presort=False, tri_off_host=None, node_features=None):
         """points: torch tensor [n_points_total, 3] float64 (host pinned or device), meshes in the
         order targets then sources; tris: int32 [n_tris_total, 3] with GLOBAL vertex ids;
         mesh_off_host: int32 [2P+1].  Returns a dict of device tensors + host metadata.
@@ -100,7 +147,20 @@ class SpectralBatch:
         new device tensor before anything else; ``points`` is never modified and ``icp_matrices`` holds the (P, 4, 4)
         matrices.  ICP needs each mesh's triangle range: ``tri_off_host`` int [2P+1], or else it is derived from
         ``tris``, which must then be grouped by mesh in mesh order as ``pack_meshes`` makes them (``ValueError``
-        otherwise; for device ``tris`` the check reads one small result back to the host)."""
+        otherwise; for device ``tris`` the check reads one small result back to the host).
+
+        ``node_features``: the mesh point scalars named by ``list_features_to_get_from_mesh``, host or device
+        [n_points_total][len(list_features_to_get_from_mesh)] in the column order of the names (``run_meshes`` fills it);
+        required when names are given.  With features on, ``node_features`` in the result is the normalised [n_points]
+        [f] block (curvature columns first) and ``coords`` the extended coordinates."""
+        n_mesh_feats = len(self.list_features_to_get_from_mesh)
+        if n_mesh_feats:
+            n_total = int(np.asarray(mesh_off_host)[-1])
+            if node_features is None:
+                raise ValueError("list_features_to_get_from_mesh names %d mesh scalar(s): pass them as node_features "
+                                 "[n_points][%d] (run_meshes does)" % (n_mesh_feats, n_mesh_feats))
+            if tuple(node_features.shape) != (n_total, n_mesh_feats):
+                raise ValueError("node_features must be [%d][%d], got %s" % (n_total, n_mesh_feats, tuple(node_features.shape)))
         torch = _lib.require_cuda()
         P = int(n_pairs)
         ev = []
@@ -116,7 +176,11 @@ class SpectralBatch:
         if self.icp_register_first:
             points, tris, icp_mats = self._icp(points, tris, mesh_off_host, P, tri_off_host)
             mark("icp")
-        g = DeviceGraph.from_device(points, tris, mesh_off_host)
+        feats, edge_points = None, None
+        if self.features_on:
+            points, tris, feats, edge_points = self._node_features(points, tris, mesh_off_host, node_features)
+            mark("features")
+        g = DeviceGraph.from_device(points, tris, mesh_off_host, edge_points)
         mark("laplacian")
         n, ns = self.n, self.ns
         nt_total = int(g.mesh_off_host[P])
@@ -168,6 +232,15 @@ class SpectralBatch:
         g.flip_permute(vecs, dst, src, sign)
         coords = g.spectral_coords(vecs, weights, ns)
         mark("eigsort")
+        if self.features_as_coords or self.include_points_as_features:  # focusr.py:218-295, in Focusr's order
+            smoothed_f = None
+            if self.features_as_coords:  # focusr_mean_filter smooths up to 8 columns per call
+                parts = [g.mean_filter(feats[:, a:a + 8].contiguous(), self.feature_smoothing_iterations)
+                         for a in range(0, self.n_node_features, 8)]
+                smoothed_f = parts[0] if len(parts) == 1 else torch.cat(parts, dim=1)
+            coords = _device.feature_coords(coords, smoothed_f, g.points, g.mesh_off, self.include_points_as_features,
+                                            self.norm_physical_and_spectral)
+            mark("feature_coords")
 
         dev = g.device
         ref_off = g.mesh_off[: P + 1].contiguous()
@@ -208,7 +281,37 @@ class SpectralBatch:
                     source_projected_on_target=src_proj[nt_total:], final_idx=idx1[:, 0], knn3_idx=idx3,
                     knn3_dist=dist3, weighted_avg_transformed_points=weighted,
                     nearest_neighbor_transformed_points=nearest, idx_t=idx_t, idx_s=idx_s, costs=costs,
-                    eig_vecs_presort=presort, cpd_idx=cpd_idx, coords_b4_reg=coords_b4_reg, icp_matrices=icp_mats)
+                    eig_vecs_presort=presort, cpd_idx=cpd_idx, coords_b4_reg=coords_b4_reg, icp_matrices=icp_mats,
+                    node_features=feats)
+
+    def _node_features(self, points, tris, mesh_off_host, node_features):
+        """graph.py:84-142,166-175 for every mesh at once: curvature of the (moved) points in one focusr_curvatures call
+        over the whole batch (it synchronises once, for its index check), the mesh scalars behind it, then
+        focusr_node_features.  Returns the device points and triangles, the normalised features [n_points][f] and the
+        edge points [n_points][3 + f] (None unless the features go into the edge weights)."""
+        torch = _lib.require_cuda()
+        lib = _lib.load()
+        dev = torch.device("cuda", torch.cuda.current_device())
+        pts = points.to(dev, non_blocking=True).contiguous()
+        tr = tris.to(dev, non_blocking=True).contiguous()
+        n, nf = int(pts.shape[0]), int(tr.shape[0])
+        raw = torch.empty((n, self.n_node_features), dtype=torch.float64, device=dev)
+        nc = len(self.curvature_columns)
+        if nc:
+            curv = torch.empty((2, n), dtype=torch.float64, device=dev)
+            ws_bytes = int(lib.focusr_curvature_workspace_bytes(n, nf))
+            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+            _lib.call("focusr_curvatures", _lib.ptr(pts), _lib.ptr(tr), n, nf, None, None, _lib.ptr(curv[0]),
+                      _lib.ptr(curv[1]), _lib.ptr(ws), ws_bytes, _lib.stream_ptr())
+            for k, c in enumerate(self.curvature_columns):
+                raw[:, k] = curv[0 if c == "minimum" else 1]
+        if nc < self.n_node_features:
+            raw[:, nc:] = torch.as_tensor(node_features, dtype=torch.float64).to(dev, non_blocking=True)
+        mesh_off = torch.from_numpy(np.ascontiguousarray(mesh_off_host, dtype=np.int32)).to(dev, non_blocking=True)
+        feats, edge_points = _device.node_features(raw, pts, mesh_off, self.norm_node_features_std,
+                                                   self.norm_node_features_cap_std, self.norm_node_features_0_1,
+                                                   want_edge_points=self.features_in_adjacency)
+        return pts, tr, feats, edge_points
 
     def _icp(self, points, tris, mesh_off_host, P, tri_off_host):
         """focusr.py:110-131 for every pair at once (``focusr_icp_batch``): returns the device points with each pair's
@@ -454,8 +557,15 @@ class SpectralBatch:
         return pts, tris, off, len(targets)
 
     def run_meshes(self, targets, sources, **kw):
-        """Convenience: lists of PolyData-like meshes (``.points``, ``.tris``)."""
+        """Convenience: lists of PolyData-like meshes (``.points``, ``.tris``); the point scalars named by
+        ``list_features_to_get_from_mesh`` are read from the meshes (``Exception`` for a missing name, as graph.py)."""
         pts, tris, off, n_pairs = self.pack_meshes(targets, sources)
+        if self.list_features_to_get_from_mesh and "node_features" not in kw:
+            import torch
+
+            kw["node_features"] = torch.from_numpy(np.ascontiguousarray(np.stack(
+                [np.concatenate([mesh_point_scalars(m, name).reshape(-1) for m in list(targets) + list(sources)])
+                 for name in self.list_features_to_get_from_mesh], axis=1)))
         tri_off = np.zeros(len(targets) + len(sources) + 1, dtype=np.int32)
         tri_off[1:] = np.cumsum([m.tris.shape[0] for m in list(targets) + list(sources)])
         kw.setdefault("tri_off_host", tri_off)

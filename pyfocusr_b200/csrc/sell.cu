@@ -1061,6 +1061,8 @@ int focusr_mean_filter(const int* row_ptr, const int* cols, const double* weight
       e = launch_pdl(k_mean_filter<3>, grid, block, stream, row_ptr, cols, weights, degree, row_begin, row_end, src, dst, 3);
     else if (n_cols == 1)
       e = launch_pdl(k_mean_filter<1>, grid, block, stream, row_ptr, cols, weights, degree, row_begin, row_end, src, dst, 1);
+    else if (n_cols == 2)  // the two curvature columns of node features (SpectralBatch)
+      e = launch_pdl(k_mean_filter<2>, grid, block, stream, row_ptr, cols, weights, degree, row_begin, row_end, src, dst, 2);
     else
       e = launch_pdl(k_mean_filter<0>, grid, block, stream, row_ptr, cols, weights, degree, row_begin, row_end, src, dst, n_cols);
     FB_CUDA(e);
