@@ -281,6 +281,21 @@ int focusr_knn(const double* refs, int ld_refs, const int* ref_off, int n_refs_t
                long long* idx, double* dist, void* workspace, size_t workspace_bytes,
                focusr_stream_t stream);
 
+/* K4 against shared reference segments (many sources against one template): query segment s searches
+ * refs[ref_off[r]..ref_off[r+1]) with r = ref_seg[s] (device int32 [n_query_segments]; `ref_seg_host` is its host copy,
+ * checked to lie in [0, n_ref_segments)).  Reference segments are n_ref_segments, possibly fewer than the query
+ * segments, and need not all be used.  Each reference segment is Morton-sorted and tiled once, in its own bounding box,
+ * and its tiles serve every query segment mapped to it.  `max_refs_per_segment` bounds every reference segment.  Same
+ * arithmetic, tie rule and brute-force rule as focusr_knn: the output is bit-identical to focusr_knn on a copy of
+ * reference segment ref_seg[s] for every query segment s.  workspace = NULL selects plain brute force. */
+size_t focusr_knn_mapped_workspace_bytes(int n_refs_total, int n_queries_total, int n_ref_segments, int dim);
+int focusr_knn_mapped(const double* refs, int ld_refs, const int* ref_off, int n_refs_total,
+                      int n_ref_segments, int max_refs_per_segment, const double* queries, int ld_queries,
+                      const int* query_off, int n_queries_total, int max_queries_per_segment,
+                      int n_query_segments, const int* ref_seg, const int* ref_seg_host, int dim, int k,
+                      long long* idx, double* dist, void* workspace, size_t workspace_bytes,
+                      focusr_stream_t stream);
+
 /* The distance matrix of the 'hungarian' correspondence (focusr.py:340-349: scipy cdist(spectral_pts,
  * target_pts), euclidean): out [n_a][n_b] = |a_i - b_j|_2. */
 int focusr_cdist(const double* a, int n_a, const double* b, int n_b, int dim, double* out,

@@ -260,6 +260,38 @@ def knn(refs, queries, k=1, ref_off=None, query_off=None, max_queries=None, max_
     return idx, dist
 
 
+def knn_mapped(refs, queries, ref_off, query_off, ref_seg, k=1, max_queries=None, max_refs=None, want_dist=True,
+               brute_force=False):
+    """Exact k-NN against shared reference segments (``focusr_knn_mapped``): query segment s (``query_off``, device
+    int32) searches reference segment ``ref_seg[s]`` (``ref_off``, device int32; ``ref_seg`` host ints).  Indices are
+    local to the reference segment; the result equals :func:`knn` on a copy of reference segment ``ref_seg[s]`` for
+    every query segment.  ``max_refs`` must bound every reference segment."""
+    torch = _torch()
+    lib = _lib.load()
+    dev = refs.device
+    nq, dim, nr = int(queries.shape[0]), int(queries.shape[1]), int(refs.shape[0])
+    seg_host = np.ascontiguousarray(ref_seg, dtype=np.int32).reshape(-1)
+    n_ref_seg, n_q_seg = int(ref_off.shape[0]) - 1, int(query_off.shape[0]) - 1
+    if seg_host.size != n_q_seg:
+        raise ValueError("knn_mapped: ref_seg needs one entry per query segment (%d), got %d" % (n_q_seg, seg_host.size))
+    if max_refs is None:
+        max_refs = int(torch.diff(ref_off).max().item())
+    if max_queries is None:
+        max_queries = int(torch.diff(query_off).max().item())
+    seg_dev = torch.from_numpy(seg_host).to(dev, non_blocking=True)
+    idx = torch.empty((nq, k), dtype=torch.int64, device=dev)
+    dist = torch.empty((nq, k), dtype=torch.float64, device=dev) if want_dist else None
+    ws, ws_bytes = None, 0
+    if not brute_force:
+        ws_bytes = int(lib.focusr_knn_mapped_workspace_bytes(nr, nq, n_ref_seg, dim))
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    _lib.call("focusr_knn_mapped", _lib.ptr(refs), int(refs.stride(0)), _lib.ptr(ref_off), nr, n_ref_seg, int(max_refs),
+              _lib.ptr(queries), int(queries.stride(0)), _lib.ptr(query_off), nq, int(max_queries), n_q_seg,
+              _lib.ptr(seg_dev), _lib.ptr(seg_host), dim, int(k), _lib.ptr(idx), _lib.ptr(dist), _lib.ptr(ws), ws_bytes,
+              _lib.stream_ptr())
+    return idx, dist
+
+
 def cdist(a, b):
     """scipy.spatial.distance.cdist(a, b) (euclidean) on the device: [n_a][n_b] float64."""
     torch = _torch()

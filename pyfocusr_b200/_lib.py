@@ -64,6 +64,9 @@ SIGNATURES = {
                                    _vp, _sz, _vp]),
     "focusr_knn_workspace_bytes": (_sz, [_i, _i, _i, _i]),
     "focusr_knn": (_i, [_vp, _i, _vp, _i, _i, _vp, _i, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _sz, _vp]),
+    "focusr_knn_mapped_workspace_bytes": (_sz, [_i, _i, _i, _i]),
+    "focusr_knn_mapped": (_i, [_vp, _i, _vp, _i, _i, _i, _vp, _i, _vp, _i, _i, _i, _vp, _vp, _i, _i, _vp, _vp, _vp, _sz,
+                               _vp]),
     "focusr_cdist": (_i, [_vp, _i, _vp, _i, _i, _vp, _vp]),
     "focusr_lsap_workspace_bytes": (_sz, [_i]),
     "focusr_lsap": (_i, [_vp, _i, _i, _vp, _vp, _vp, _sz, _vp]),

@@ -9,7 +9,10 @@ of the vertices and the download of the correspondences except the eigensolver's
 (a few hundred Ritz values and residuals per outer iteration) and, with node features on, the one synchronise of
 ``focusr_curvatures`` (its triangle-index check).
 
-Mesh order inside the batch graph: targets 0..P-1, then sources 0..P-1.
+Mesh order inside the batch graph: targets 0..P-1, then sources 0..P-1.  With ``run(..., target_of_pair=...)`` (many
+sources against a few templates) the batch graph holds T distinct targets, then the P sources, and pair p is target
+``target_of_pair[p]`` with source p: each target is built, solved and smoothed once, and the results are returned in the
+pair layout (target copy p, then source p) of the batch with every target repeated once per pair.
 """
 from __future__ import annotations
 
@@ -26,6 +29,72 @@ __all__ = ["SpectralBatch"]
 # graph.py:11-15 (features_dictionary): the focusr_curvatures outputs each name contributes, in order
 CURVATURE_FEATURES = {"curvature": ("minimum", "maximum"), "min_curvature": ("minimum",), "max_curvature": ("maximum",)}
 MAX_KNN_DIM, MAX_CPD_DIM = 32, 16  # focusr_knn, focusr_cpd_*
+
+
+def shared_targets(target_of_pair, n_meshes, n_pairs):
+    """Checks ``target_of_pair`` of a batch of ``n_meshes`` meshes (T targets, then ``n_pairs`` sources) and returns it as
+    int32 [P] with T.  ``ValueError`` unless it has one integer per pair, T >= 1, every value lies in [0, T) and every
+    target is used by some pair."""
+    P = int(n_pairs)
+    T = int(n_meshes) - P
+    top = np.asarray(target_of_pair)
+    if top.ndim != 1 or top.size != P:
+        raise ValueError("target_of_pair needs one entry per pair (%d), got shape %s" % (P, top.shape))
+    if P < 1 or T < 1:
+        raise ValueError("a batch with target_of_pair needs at least one pair and one target (mesh layout: T targets, then "
+                         "%d sources; %d meshes given)" % (P, n_meshes))
+    if top.dtype.kind not in "iu":
+        if top.dtype.kind != "f" or not np.all(np.isfinite(top)) or not np.all(top == np.round(top)):
+            raise ValueError("target_of_pair must hold integers")
+    top = top.astype(np.int64)
+    bad = np.nonzero((top < 0) | (top >= T))[0]
+    if bad.size:
+        raise ValueError("target_of_pair[%d] = %d lies outside [0, %d)" % (bad[0], top[bad[0]], T))
+    unused = np.setdiff1d(np.arange(T), top)
+    if unused.size:
+        raise ValueError("target(s) %s are used by no pair: a batch holds only the targets its pairs use" % unused[:16].tolist())
+    return top.astype(np.int32), T
+
+
+class PairLayout:
+    """The pair layout of a shared-target batch: 2P meshes, copy p of target ``target_of_pair[p]``, then source p.  It
+    stands in for the batch's ``DeviceGraph`` in the stages that work pair by pair (eigsort, spectral and feature
+    coordinates, CPD, the first KNN): same attributes (``mesh_off`` / ``mesh_off_host``, ``n_meshes``, ``n_points``,
+    ``max_mesh_points``, ``points``, ``device``) and the same column methods, but no Laplacian of its own.  ``rows``
+    gathers per-vertex rows of the batch graph into this layout (``focusr_gather_rows``)."""
+
+    flip_permute = DeviceGraph.flip_permute
+    spectral_coords = DeviceGraph.spectral_coords
+
+    def __init__(self, g, target_of_pair):
+        torch = _lib.require_cuda()
+        P = int(target_of_pair.size)
+        T = g.n_meshes - P
+        real_off = g.mesh_off_host.astype(np.int64)
+        self.mesh_of = np.concatenate([target_of_pair, np.arange(T, T + P)]).astype(np.int64)  # batch mesh of each mesh
+        sizes = np.diff(real_off)[self.mesh_of]
+        self.mesh_off_host = np.zeros(2 * P + 1, dtype=np.int32)
+        self.mesh_off_host[1:] = np.cumsum(sizes)
+        self.n_meshes = 2 * P
+        self.n_points = int(self.mesh_off_host[-1])
+        self.max_mesh_points = int(sizes.max())
+        self.device = dev = g.device
+        self.mesh_off = torch.from_numpy(self.mesh_off_host).to(dev, non_blocking=True)
+        self.mesh_map = torch.from_numpy(self.mesh_of).to(dev, non_blocking=True)
+        # batch row of every row of this layout: its mesh's shift, repeated over the mesh's rows, plus the row itself
+        shift = torch.from_numpy(real_off[self.mesh_of] - self.mesh_off_host[:-1]).to(dev, non_blocking=True)
+        self.row_map = torch.arange(self.n_points, dtype=torch.int64, device=dev) + torch.repeat_interleave(
+            shift, torch.from_numpy(sizes).to(dev, non_blocking=True), output_size=self.n_points)
+        self.points = self.rows(g.points)
+
+    def rows(self, values, n_rows=None):
+        """Per-vertex rows [n_points of the batch][c] -> the first ``n_rows`` rows of this layout (default: all)."""
+        idx = self.row_map if n_rows is None else self.row_map[:n_rows]
+        return _device.gather_rows(values.contiguous(), idx)
+
+    def meshes(self, values):
+        """Per-mesh rows [batch meshes][c] -> [2P][c]."""
+        return _device.gather_rows(values.contiguous(), self.mesh_map)
 
 
 def mesh_point_scalars(mesh, name):
@@ -138,7 +207,7 @@ class SpectralBatch:
 
     # ------------------------------------------------------------------------------------------
     def run(self, points, tris, mesh_off_host, n_pairs, idx_t=None, idx_s=None, record_events=False,
-            keep_presort=False, tri_off_host=None, node_features=None):
+            keep_presort=False, tri_off_host=None, node_features=None, target_of_pair=None):
         """points: torch tensor [n_points_total, 3] float64 (host pinned or device), meshes in the
         order targets then sources; tris: int32 [n_tris_total, 3] with GLOBAL vertex ids;
         mesh_off_host: int32 [2P+1].  Returns a dict of device tensors + host metadata.
@@ -152,7 +221,23 @@ class SpectralBatch:
         ``node_features``: the mesh point scalars named by ``list_features_to_get_from_mesh``, host or device
         [n_points_total][len(list_features_to_get_from_mesh)] in the column order of the names (``run_meshes`` fills it);
         required when names are given.  With features on, ``node_features`` in the result is the normalised [n_points]
-        [f] block (curvature columns first) and ``coords`` the extended coordinates."""
+        [f] block (curvature columns first) and ``coords`` the extended coordinates.
+
+        ``target_of_pair`` (int [P]): many sources against shared targets.  The mesh layout is then T targets, then the P
+        sources (T = len(mesh_off_host) - 1 - n_pairs), and pair p is target ``target_of_pair[p]`` with source p.  Each
+        target's Laplacian, eigenpairs, features and 300 smoothing passes are computed once; the results are gathered
+        into the pair layout (target copy p, then source p), and every key equals, bit for bit, that of ``run`` on the
+        batch with each target repeated once per pair, except ``graph`` and ``eigs_info``, which describe the T + P meshes
+        built and solved.  ``pair_mesh_off`` holds the pair layout's mesh offsets (with ``target_of_pair=None``: those of
+        ``graph``).  ``node_features`` and ``tri_off_host`` follow the T + P layout.  ``ValueError`` for a target outside
+        [0, T), a target no pair uses, or ``icp_reg_target_to_source`` with ICP on and a target shared by two pairs."""
+        P = int(n_pairs)
+        top = None
+        if target_of_pair is not None:
+            top, T = shared_targets(target_of_pair, np.asarray(mesh_off_host).size - 1, P)
+            if self.icp_register_first and self.icp_reg_target_to_source and np.unique(top).size < P:
+                raise ValueError("icp_reg_target_to_source moves each pair's target onto its source: a target shared by "
+                                 "several pairs would move differently for each of them")
         n_mesh_feats = len(self.list_features_to_get_from_mesh)
         if n_mesh_feats:
             n_total = int(np.asarray(mesh_off_host)[-1])
@@ -162,7 +247,6 @@ class SpectralBatch:
             if tuple(node_features.shape) != (n_total, n_mesh_feats):
                 raise ValueError("node_features must be [%d][%d], got %s" % (n_total, n_mesh_feats, tuple(node_features.shape)))
         torch = _lib.require_cuda()
-        P = int(n_pairs)
         ev = []
 
         def mark(name):
@@ -174,7 +258,7 @@ class SpectralBatch:
         mark("start")
         icp_mats = None
         if self.icp_register_first:
-            points, tris, icp_mats = self._icp(points, tris, mesh_off_host, P, tri_off_host)
+            points, tris, icp_mats = self._icp(points, tris, mesh_off_host, P, tri_off_host, top)
             mark("icp")
         feats, edge_points = None, None
         if self.features_on:
@@ -183,7 +267,8 @@ class SpectralBatch:
         g = DeviceGraph.from_device(points, tris, mesh_off_host, edge_points)
         mark("laplacian")
         n, ns = self.n, self.ns
-        nt_total = int(g.mesh_off_host[P])
+        nt_mesh = P if top is None else T  # targets in the batch graph
+        nt_total = int(g.mesh_off_host[nt_mesh])
         smoothed_t, side = None, None
         if self.overlap_smoothing:
             main = torch.cuda.current_stream()
@@ -202,19 +287,31 @@ class SpectralBatch:
             if info is None:
                 raise
             bad = np.nonzero(info["status"] != 0)[0]
-            raise RuntimeError("eigensolve failed for %d of %d meshes: %s (mesh m is the %s of pair m %% %d); the other "
-                               "meshes of the batch were solved -- drop the named pairs and rerun" % (
-                                   bad.size, 2 * P, ", ".join("mesh %d: %s" % (m, _device.EIG_STATUS.get(int(info["status"][m]), "?"))
-                                                              for m in bad[:16]), "target if m < %d else source" % P, P)) from exc
+            if top is None:
+                raise RuntimeError("eigensolve failed for %d of %d meshes: %s (mesh m is the %s of pair m %% %d); the other "
+                                   "meshes of the batch were solved -- drop the named pairs and rerun" % (
+                                       bad.size, 2 * P, ", ".join("mesh %d: %s" % (m, _device.EIG_STATUS.get(int(info["status"][m]), "?"))
+                                                                  for m in bad[:16]), "target if m < %d else source" % P, P)) from exc
+            raise RuntimeError("eigensolve failed for %d of %d meshes: %s; the other meshes of the batch were solved -- drop "
+                               "the named pairs and rerun" % (bad.size, T + P, ", ".join(
+                                   "%s: %s" % (self._mesh_pairs(m, top), _device.EIG_STATUS.get(int(info["status"][m]), "?"))
+                                   for m in bad[:16]))) from exc
         n_found = info["n_found"]
         if int(n_found.min()) < n:
             short = np.nonzero(n_found < n)[0]
-            raise RuntimeError("meshes %s returned fewer than %d eigenpairs (pairs %s)" % (
-                short[:16].tolist(), n, sorted(set(int(m) % P for m in short[:16]))))
+            if top is None:
+                raise RuntimeError("meshes %s returned fewer than %d eigenpairs (pairs %s)" % (
+                    short[:16].tolist(), n, sorted(set(int(m) % P for m in short[:16]))))
+            raise RuntimeError("fewer than %d eigenpairs for %s" % (n, "; ".join(self._mesh_pairs(m, top) for m in short[:16])))
         g.normalize_columns(vecs, n_found)
         mark("eigensolve")
+        pg = g  # the graph of the pair stages: the batch graph itself, or its pair layout
+        if top is not None:  # gather the target rows into the pair layout; the sources keep their rows
+            pg = PairLayout(g, top)
+            vecs, vals, n_found = pg.rows(vecs), pg.meshes(vals), n_found[pg.mesh_of]
+            mark("pair_layout")
 
-        off = g.mesh_off_host
+        off = pg.mesh_off_host
         sizes = np.diff(off)
         if idx_t is None:
             rng = np.random.RandomState(self.seed)
@@ -222,15 +319,15 @@ class SpectralBatch:
             idx_s = self.sample_indices(sizes[P:], rng)
         t_mesh = np.arange(P, dtype=np.int32)
         s_mesh = np.arange(P, 2 * P, dtype=np.int32)
-        ch, chf, cs, csf, _ = _device.eigsort_costs(g, vecs, t_mesh, s_mesh, idx_t, idx_s, n)
+        ch, chf, cs, csf, _ = _device.eigsort_costs(pg, vecs, t_mesh, s_mesh, idx_t, idx_s, n)
         # n x n decisions per pair (eigsort.py:66-122, 142-160; focusr.py:459-490) on the device: c_lambda, min(c, c_f),
         # the assignment (scipy's algorithm and tie rules), flips, column moves and spectral weights -- no host visit
         Q, dst, src, sign, weights, decide_status = _device.eigsort_decide(
-            g, vals, n_found, t_mesh, s_mesh, (ch, chf, cs, csf), n, ns, self.target_as_reference, self.weighted)
+            pg, vals, n_found, t_mesh, s_mesh, (ch, chf, cs, csf), n, ns, self.target_as_reference, self.weighted)
         costs = (ch, chf, cs, csf)
         presort = vecs.clone() if keep_presort else None
-        g.flip_permute(vecs, dst, src, sign)
-        coords = g.spectral_coords(vecs, weights, ns)
+        pg.flip_permute(vecs, dst, src, sign)
+        coords = pg.spectral_coords(vecs, weights, ns)
         mark("eigsort")
         if self.features_as_coords or self.include_points_as_features:  # focusr.py:218-295, in Focusr's order
             smoothed_f = None
@@ -238,27 +335,35 @@ class SpectralBatch:
                 parts = [g.mean_filter(feats[:, a:a + 8].contiguous(), self.feature_smoothing_iterations)
                          for a in range(0, self.n_node_features, 8)]
                 smoothed_f = parts[0] if len(parts) == 1 else torch.cat(parts, dim=1)
-            coords = _device.feature_coords(coords, smoothed_f, g.points, g.mesh_off, self.include_points_as_features,
+                if top is not None:
+                    smoothed_f = pg.rows(smoothed_f)
+            coords = _device.feature_coords(coords, smoothed_f, pg.points, pg.mesh_off, self.include_points_as_features,
                                             self.norm_physical_and_spectral)
             mark("feature_coords")
 
         dev = g.device
-        ref_off = g.mesh_off[: P + 1].contiguous()
-        qry_off = (g.mesh_off[P:] - nt_total).contiguous()
+        nt_pair = int(off[P])
+        ref_off = pg.mesh_off[: P + 1].contiguous()
+        qry_off = (pg.mesh_off[P:] - nt_pair).contiguous()
         max_q, max_r = int(sizes[P:].max()), int(sizes[:P].max())
         cpd_idx, coords_b4_reg = None, None
         if self.registration == "b200":  # register every pair's target coordinates onto its source's
             coords_b4_reg = coords.clone()
             cpd_idx = self._register_pairs(coords, off, P, sizes)
             mark("cpd")
-        idx0, _ = _device.knn(coords[:nt_total], coords[nt_total:], k=1, ref_off=ref_off, query_off=qry_off,
+        idx0, _ = _device.knn(coords[:nt_pair], coords[nt_pair:], k=1, ref_off=ref_off, query_off=qry_off,
                               max_queries=max_q, max_refs=max_r, want_dist=False)
         mark("knn_initial")
         if side is not None:
             torch.cuda.current_stream().wait_stream(side)
         else:
             smoothed_t = g.mean_filter(g.points, self.graph_smoothing_iterations, 0, nt_total)
-        base_q = torch.repeat_interleave(g.mesh_off[:P], torch.from_numpy(sizes[P:].astype(np.int64)).to(dev)).to(torch.int32)
+        if top is None:
+            base_q = torch.repeat_interleave(g.mesh_off[:P], torch.from_numpy(sizes[P:].astype(np.int64)).to(dev)).to(torch.int32)
+        else:  # the first row of each pair's target in the batch graph
+            base_q = torch.repeat_interleave(torch.from_numpy(g.mesh_off_host[top]).to(dev, non_blocking=True),
+                                             torch.from_numpy(sizes[P:].astype(np.int64)).to(dev, non_blocking=True),
+                                             output_size=g.n_points - nt_total)
         staged = torch.empty_like(g.points)
         _lib.call("focusr_gather_rows", _lib.ptr(smoothed_t), _lib.ptr(idx0), _lib.ptr(base_q), g.n_points - nt_total, 3,
                   _lib.ptr(staged[nt_total:]), _lib.stream_ptr())
@@ -266,23 +371,39 @@ class SpectralBatch:
         mark("smoothing")
         # one k=3 search serves both focusr.py:391-392 (k=1: its first column, same distances and tie
         # rule) and focusr.py:409-413 (k=3)
-        idx3, dist3 = _device.knn(smoothed_t[:nt_total], src_proj[nt_total:], k=3, ref_off=ref_off, query_off=qry_off,
-                                  max_queries=max_q, max_refs=max_r)
+        if top is None:
+            idx3, dist3 = _device.knn(smoothed_t[:nt_total], src_proj[nt_total:], k=3, ref_off=ref_off, query_off=qry_off,
+                                      max_queries=max_q, max_refs=max_r)
+        else:  # each target's Morton sort and tiles serve all of its pairs
+            idx3, dist3 = _device.knn_mapped(smoothed_t[:nt_total], src_proj[nt_total:], g.mesh_off[: T + 1].contiguous(),
+                                             (g.mesh_off[T:] - nt_total).contiguous(), top, k=3, max_queries=max_q,
+                                             max_refs=int(np.diff(g.mesh_off_host[: T + 1]).max()))
         idx1 = idx3[:, :1]
         weighted = _device.weighted_positions(idx3, dist3, g.points, base_q)
         nearest = _device.gather_rows(g.points, idx1[:, 0].contiguous(), base_q)
         mark("knn_final")
+        smoothed_tc = smoothed_t[:nt_total] if top is None else pg.rows(smoothed_t, nt_pair)
+        if top is not None and feats is not None:
+            feats = pg.rows(feats)
         if record_events:
             torch.cuda.synchronize()
             self.timings = {ev[i][0]: ev[i - 1][1].elapsed_time(ev[i][1]) for i in range(1, len(ev))}
         return dict(graph=g, eig_vals=vals, eig_vecs=vecs, eigs_info=info, Q=Q, spectral_weights=weights[:P],
-                    eigsort_status=decide_status,
-                    coords=coords, initial_idx=idx0[:, 0], smoothed_target_coords=smoothed_t[:nt_total],
+                    eigsort_status=decide_status, pair_mesh_off=off,
+                    coords=coords, initial_idx=idx0[:, 0], smoothed_target_coords=smoothed_tc,
                     source_projected_on_target=src_proj[nt_total:], final_idx=idx1[:, 0], knn3_idx=idx3,
                     knn3_dist=dist3, weighted_avg_transformed_points=weighted,
                     nearest_neighbor_transformed_points=nearest, idx_t=idx_t, idx_s=idx_s, costs=costs,
                     eig_vecs_presort=presort, cpd_idx=cpd_idx, coords_b4_reg=coords_b4_reg, icp_matrices=icp_mats,
                     node_features=feats)
+
+    @staticmethod
+    def _mesh_pairs(m, top):
+        """Mesh m of a shared-target batch graph named by the pairs it serves."""
+        T = int(top.max()) + 1
+        if m < T:
+            return "target %d (pairs %s)" % (m, np.nonzero(top == m)[0].tolist())
+        return "source of pair %d" % (m - T)
 
     def _node_features(self, points, tris, mesh_off_host, node_features):
         """graph.py:84-142,166-175 for every mesh at once: curvature of the (moved) points in one focusr_curvatures call
@@ -313,9 +434,10 @@ class SpectralBatch:
                                                    want_edge_points=self.features_in_adjacency)
         return pts, tr, feats, edge_points
 
-    def _icp(self, points, tris, mesh_off_host, P, tri_off_host):
+    def _icp(self, points, tris, mesh_off_host, P, tri_off_host, target_of_pair=None):
         """focusr.py:110-131 for every pair at once (``focusr_icp_batch``): returns the device points with each pair's
-        moving mesh registered onto its fixed one (a new tensor), the device triangles and the (P, 4, 4) matrices."""
+        moving mesh registered onto its fixed one (a new tensor), the device triangles and the (P, 4, 4) matrices.  With
+        ``target_of_pair`` pair p is batch mesh ``target_of_pair[p]`` with mesh T + p."""
         torch = _lib.require_cuda()
         off = np.ascontiguousarray(mesh_off_host, dtype=np.int32)
         if tri_off_host is None:
@@ -324,6 +446,9 @@ class SpectralBatch:
         pts = points.to(dev, non_blocking=True).contiguous()
         tr = tris.to(dev, non_blocking=True).contiguous()
         targets, sources = np.arange(P, dtype=np.int32), np.arange(P, 2 * P, dtype=np.int32)
+        if target_of_pair is not None:
+            T = off.size - 1 - P
+            targets, sources = np.asarray(target_of_pair, dtype=np.int32), np.arange(T, T + P, dtype=np.int32)
         fixed, moving = (sources, targets) if self.icp_reg_target_to_source else (targets, sources)
         mats, moved = _device.icp_batch_device(pts, tr, off, tri_off_host, fixed, moving, max_iterations=100,
                                                max_landmarks=1000, similarity=self.icp_registration_mode == "similarity")
@@ -540,13 +665,18 @@ class SpectralBatch:
 
     # ------------------------------------------------------------------------------------------
     @staticmethod
-    def pack_meshes(targets, sources):
+    def pack_meshes(targets, sources, target_of_pair=None):
         """Lists of PolyData-like meshes (``.points``, ``.tris``) -> ``(points, tris, mesh_off_host, n_pairs)`` of ``run``
-        (host tensors; targets first, then sources; triangle vertex ids made global)."""
+        (host tensors; targets first, then sources; triangle vertex ids made global).  With ``target_of_pair`` (int [P],
+        one entry per source) the targets are the T shared ones, pair p being ``targets[target_of_pair[p]]`` with
+        ``sources[p]``; without it, pair p is ``targets[p]`` with ``sources[p]``."""
         import torch
 
-        if len(targets) != len(sources) or not targets:
-            raise ValueError("need as many source meshes as target meshes (at least one pair)")
+        if target_of_pair is None:
+            if len(targets) != len(sources) or not targets:
+                raise ValueError("need as many source meshes as target meshes (at least one pair)")
+        else:
+            shared_targets(target_of_pair, len(targets) + len(sources), len(sources))
         meshes = list(targets) + list(sources)
         sizes = [m.points.shape[0] for m in meshes]
         off = np.zeros(len(meshes) + 1, dtype=np.int32)
@@ -554,12 +684,15 @@ class SpectralBatch:
         pts = torch.from_numpy(np.ascontiguousarray(np.concatenate([m.points for m in meshes])))
         tris = torch.from_numpy(np.ascontiguousarray(np.concatenate(
             [m.tris.astype(np.int64) + int(o) for m, o in zip(meshes, off[:-1])]).astype(np.int32)))
-        return pts, tris, off, len(targets)
+        return pts, tris, off, len(sources)
 
-    def run_meshes(self, targets, sources, **kw):
+    def run_meshes(self, targets, sources, target_of_pair=None, **kw):
         """Convenience: lists of PolyData-like meshes (``.points``, ``.tris``); the point scalars named by
-        ``list_features_to_get_from_mesh`` are read from the meshes (``Exception`` for a missing name, as graph.py)."""
-        pts, tris, off, n_pairs = self.pack_meshes(targets, sources)
+        ``list_features_to_get_from_mesh`` are read from the meshes (``Exception`` for a missing name, as graph.py).
+        ``target_of_pair``: as in ``pack_meshes`` and ``run`` (many sources against shared targets)."""
+        pts, tris, off, n_pairs = self.pack_meshes(targets, sources, target_of_pair)
+        if target_of_pair is not None:
+            kw["target_of_pair"] = target_of_pair
         if self.list_features_to_get_from_mesh and "node_features" not in kw:
             import torch
 

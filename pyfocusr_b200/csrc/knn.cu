@@ -24,8 +24,8 @@ constexpr int KNN_MAX_K = 8;
 template <int D, int K>
 __global__ void __launch_bounds__(KNN_THREADS)
 k_knn(const double* __restrict__ refs, int ld_refs, const int* __restrict__ ref_off,
-      const double* __restrict__ queries, int ld_queries, const int* __restrict__ query_off, int dim_rt,
-      int k_rt, long long* __restrict__ idx, double* __restrict__ dist) {
+      const int* __restrict__ ref_seg, const double* __restrict__ queries, int ld_queries,
+      const int* __restrict__ query_off, int dim_rt, int k_rt, long long* __restrict__ idx, double* __restrict__ dist) {
   extern __shared__ double tile[];  // [KNN_TILE][dim]
   const int dim = D > 0 ? D : dim_rt;
   const int kk = K > 0 ? K : k_rt;
@@ -35,7 +35,8 @@ k_knn(const double* __restrict__ refs, int ld_refs, const int* __restrict__ ref_
   const int q0 = query_off[seg] + blockIdx.x * KNN_THREADS;
   const int q1 = query_off[seg + 1];
   if (q0 >= q1) return;
-  const int rbeg = ref_off[seg], rend = ref_off[seg + 1];
+  const int rseg = ref_seg ? ref_seg[seg] : seg;
+  const int rbeg = ref_off[rseg], rend = ref_off[rseg + 1];
   const int q = q0 + threadIdx.x;
   const bool valid = q < q1;
   double qc[DM];
@@ -93,7 +94,7 @@ k_knn(const double* __restrict__ refs, int ld_refs, const int* __restrict__ ref_
 
 int launch_knn(const double* refs, int ld_refs, const int* ref_off, const double* queries, int ld_queries,
                const int* query_off, int n_segments, int max_queries, int dim, int k, long long* idx,
-               double* dist, cudaStream_t stream) {
+               double* dist, cudaStream_t stream, const int* ref_seg) {
   if (!(dim >= 1 && dim <= KNN_MAX_DIM && k >= 1 && k <= KNN_MAX_K && n_segments > 0 && max_queries > 0)) {
     set_error("knn: need 1 <= dim <= %d, 1 <= k <= %d (got dim=%d k=%d)", KNN_MAX_DIM, KNN_MAX_K, dim, k);
     return FB_ERR_ARG;
@@ -108,7 +109,8 @@ int launch_knn(const double* refs, int ld_refs, const int* ref_off, const double
     FB_CUDA(cudaFuncSetAttribute(k_knn<0, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap));
   }
 #define FB_KNN(DD, KK) \
-  k_knn<DD, KK><<<grid, KNN_THREADS, smem, stream>>>(refs, ld_refs, ref_off, queries, ld_queries, query_off, dim, k, idx, dist)
+  k_knn<DD, KK><<<grid, KNN_THREADS, smem, stream>>>(refs, ld_refs, ref_off, ref_seg, queries, ld_queries, query_off, dim, \
+                                                     k, idx, dist)
   if (dim == 3 && k == 1)
     FB_KNN(3, 1);
   else if (dim == 3 && k == 3)
@@ -202,6 +204,29 @@ int focusr_knn(const double* refs, int ld_refs, const int* ref_off, int n_refs_t
                              idx, dist, workspace, workspace_bytes, (cudaStream_t)stream);
   return launch_knn(refs, ld_refs, ref_off, queries, ld_queries, query_off, n_segments,
                     max_queries_per_segment, dim, k, idx, dist, (cudaStream_t)stream);
+}
+
+size_t focusr_knn_mapped_workspace_bytes(int n_refs_total, int n_queries_total, int n_ref_segments, int dim) {
+  return knn_pruned_workspace_bytes(n_refs_total, n_queries_total, n_ref_segments, dim);
+}
+
+int focusr_knn_mapped(const double* refs, int ld_refs, const int* ref_off, int n_refs_total, int n_ref_segments,
+                      int max_refs_per_segment, const double* queries, int ld_queries, const int* query_off,
+                      int n_queries_total, int max_queries_per_segment, int n_query_segments, const int* ref_seg,
+                      const int* ref_seg_host, int dim, int k, long long* idx, double* dist, void* workspace,
+                      size_t workspace_bytes, focusr_stream_t stream) {
+  FB_REQUIRE(n_ref_segments > 0 && n_query_segments > 0 && n_refs_total > 0 && n_queries_total > 0, "knn_mapped: empty input");
+  FB_REQUIRE(ref_seg != nullptr && ref_seg_host != nullptr, "knn_mapped: ref_seg and its host copy are required");
+  for (int s = 0; s < n_query_segments; ++s)
+    FB_REQUIRE(ref_seg_host[s] >= 0 && ref_seg_host[s] < n_ref_segments,
+               "knn_mapped: query segment %d maps to reference segment %d, outside [0, %d)", s, ref_seg_host[s],
+               n_ref_segments);
+  if (workspace != nullptr && knn_pruned_applicable(max_refs_per_segment, max_queries_per_segment, dim, k))
+    return launch_knn_pruned(refs, ld_refs, ref_off, queries, ld_queries, query_off, n_query_segments,
+                             max_refs_per_segment, max_queries_per_segment, n_refs_total, n_queries_total, dim, k,
+                             idx, dist, workspace, workspace_bytes, (cudaStream_t)stream, n_ref_segments, ref_seg);
+  return launch_knn(refs, ld_refs, ref_off, queries, ld_queries, query_off, n_query_segments,
+                    max_queries_per_segment, dim, k, idx, dist, (cudaStream_t)stream, ref_seg);
 }
 
 int focusr_weighted_positions(const long long* idx3, const double* dist3, const double* target_points,

@@ -9,6 +9,11 @@
 // Per segment (<= 16384 points a side): one CTA sorts 64-bit (morton << 32 | index) keys with a
 // bitonic network in shared memory -- the "sort" of north_star's sort/segment-reduce vocabulary --
 // and writes the permuted reference coordinates and tile boxes.
+//
+// Mapped form (focusr_knn_mapped): query segment s searches reference segment ref_seg[s], so several query segments
+// can share one reference segment.  Each reference segment is boxed, sorted and tiled once, in a box of its own
+// references; the queries of s are keyed in the box of ref_seg[s].  ref_seg = NULL is the identity map (focusr_knn),
+// whose box is that of the segment's references and queries, as before.
 #include <limits.h>
 
 #include "common.cuh"
@@ -35,7 +40,7 @@ constexpr int PK_TQ = FB_PK_TQ;  // queries per CTA
 constexpr int PK_SORT_MAX = 16384;
 constexpr int PK_MAX_DIM = 32;
 
-// bounding box of refs U queries of each segment over the first min(dim,3) coordinates
+// bounding box of refs U queries of each segment over the first min(dim,3) coordinates (refs alone: query_off = NULL)
 __global__ void __launch_bounds__(256)
 k_pk_bbox(const double* __restrict__ refs, int ldr, const int* __restrict__ ref_off,
           const double* __restrict__ queries, int ldq, const int* __restrict__ query_off, int dim,
@@ -49,12 +54,13 @@ k_pk_bbox(const double* __restrict__ refs, int ldr, const int* __restrict__ ref_
       mn[c] = fmin(mn[c], v);
       mx[c] = fmax(mx[c], v);
     }
-  for (int r = query_off[seg] + threadIdx.x; r < query_off[seg + 1]; r += blockDim.x)
-    for (int c = 0; c < nd; ++c) {
-      const double v = queries[(size_t)r * ldq + c];
-      mn[c] = fmin(mn[c], v);
-      mx[c] = fmax(mx[c], v);
-    }
+  if (query_off)
+    for (int r = query_off[seg] + threadIdx.x; r < query_off[seg + 1]; r += blockDim.x)
+      for (int c = 0; c < nd; ++c) {
+        const double v = queries[(size_t)r * ldq + c];
+        mn[c] = fmin(mn[c], v);
+        mx[c] = fmax(mx[c], v);
+      }
   __shared__ double smn[3][256], smx[3][256];
   for (int c = 0; c < 3; ++c) {
     smn[c][threadIdx.x] = mn[c];
@@ -77,22 +83,26 @@ k_pk_bbox(const double* __restrict__ refs, int ldr, const int* __restrict__ ref_
   }
 }
 
-// grid (segments, 2): y = 0 sorts the references of the segment, y = 1 the queries.
+// grid (max(reference, query segments), 2): y = 0 sorts the references of reference segment x, y = 1 the queries of
+// query segment x, keyed in the box of the reference segment they search (ref_seg[x], or x when ref_seg is NULL).
 __global__ void __launch_bounds__(1024)
-k_pk_sort(const double* __restrict__ refs, int ldr, const int* __restrict__ ref_off,
-          const double* __restrict__ queries, int ldq, const int* __restrict__ query_off, int dim,
-          const double* __restrict__ seg_lo, const double* __restrict__ seg_inv, int p2,
+k_pk_sort(const double* __restrict__ refs, int ldr, const int* __restrict__ ref_off, int n_ref_segments,
+          const double* __restrict__ queries, int ldq, const int* __restrict__ query_off, int n_query_segments,
+          const int* __restrict__ ref_seg, int dim, const double* __restrict__ seg_lo, const double* __restrict__ seg_inv,
+          int p2,
           double* __restrict__ refs_sorted, int* __restrict__ ref_orig, int* __restrict__ q_orig,
           unsigned* __restrict__ q_key, double* __restrict__ tile_lo, double* __restrict__ tile_hi,
           unsigned* __restrict__ tile_key) {
   extern __shared__ unsigned long long keys[];
   const int seg = blockIdx.x, which = blockIdx.y;
+  if (seg >= (which == 0 ? n_ref_segments : n_query_segments)) return;
+  const int box = (which == 1 && ref_seg) ? ref_seg[seg] : seg;
   const double* src = which == 0 ? refs : queries;
   const int ld = which == 0 ? ldr : ldq;
   const int base = which == 0 ? ref_off[seg] : query_off[seg];
   const int n = (which == 0 ? ref_off[seg + 1] : query_off[seg + 1]) - base;
-  const double lo[3] = {seg_lo[3 * seg], seg_lo[3 * seg + 1], seg_lo[3 * seg + 2]};
-  const double inv[3] = {seg_inv[3 * seg], seg_inv[3 * seg + 1], seg_inv[3 * seg + 2]};
+  const double lo[3] = {seg_lo[3 * box], seg_lo[3 * box + 1], seg_lo[3 * box + 2]};
+  const double inv[3] = {seg_inv[3 * box], seg_inv[3 * box + 1], seg_inv[3 * box + 2]};
   for (int e = threadIdx.x; e < p2; e += blockDim.x) {
     unsigned long long k = ~0ull;
     if (e < n) k = ((unsigned long long)morton3(src + (size_t)(base + e) * ld, dim, lo, inv) << 32) | (unsigned)e;
@@ -172,10 +182,13 @@ unsigned long long pk_evals_read_and_maybe_reset(bool reset) {
   return v;
 }
 
-template <int D, int K>
+// grid (query blocks, query segments): query segment blockIdx.y searches reference segment ref_seg[blockIdx.y] (MAP)
+// or reference segment blockIdx.y.  MAP is a template parameter so that the identity map of focusr_knn keeps its
+// register count (a loaded segment index stays live where blockIdx.y is re-read: +8 registers at d = 3).
+template <int D, int K, bool MAP>
 __global__ void __launch_bounds__(PK_TQ)
 k_pk_search(const double* __restrict__ refs_sorted, const int* __restrict__ ref_orig, const int* __restrict__ ref_off,
-            const double* __restrict__ queries, int ldq, const int* __restrict__ query_off,
+            const int* __restrict__ ref_seg, const double* __restrict__ queries, int ldq, const int* __restrict__ query_off,
             const int* __restrict__ q_orig, const unsigned* __restrict__ q_key, const double* __restrict__ tile_lo,
             const double* __restrict__ tile_hi, const unsigned* __restrict__ tile_key, int dim_rt, int k_rt,
             long long* __restrict__ idx, double* __restrict__ dist) {
@@ -192,9 +205,10 @@ k_pk_search(const double* __restrict__ refs_sorted, const int* __restrict__ ref_
   const int qbase = query_off[seg];
   const int q0 = qbase + blockIdx.x * PK_TQ, qend = query_off[seg + 1];
   if (q0 >= qend) return;
-  const int rbase = ref_off[seg], nr = ref_off[seg + 1] - rbase;
+  const int rseg = MAP ? ref_seg[seg] : seg;
+  const int rbase = ref_off[rseg], nr = ref_off[rseg + 1] - rbase;
   const int ntiles = (nr + PK_TR - 1) / PK_TR;
-  const int tbase = rbase / PK_TR + seg;
+  const int tbase = rbase / PK_TR + rseg;
   const int pos = q0 + threadIdx.x;
   const bool valid = pos < qend;
   const int qo = valid ? q_orig[pos] : 0;
@@ -364,11 +378,12 @@ bool knn_pruned_applicable(int max_refs, int max_queries, int dim, int k) {
 int launch_knn_pruned(const double* refs, int ld_refs, const int* ref_off, const double* queries, int ld_queries,
                       const int* query_off, int n_segments, int max_refs, int max_queries, long long n_refs,
                       long long n_queries, int dim, int k, long long* idx, double* dist, void* workspace,
-                      size_t workspace_bytes, cudaStream_t stream) {
+                      size_t workspace_bytes, cudaStream_t stream, int n_ref_segments, const int* ref_seg) {
+  if (!ref_seg) n_ref_segments = n_segments;
   Carver cv(workspace, workspace_bytes);
-  const size_t tiles = (size_t)(n_refs / PK_TR) + n_segments + 1;
-  double* seg_lo = cv.take<double>(3 * (size_t)n_segments);
-  double* seg_inv = cv.take<double>(3 * (size_t)n_segments);
+  const size_t tiles = (size_t)(n_refs / PK_TR) + n_ref_segments + 1;
+  double* seg_lo = cv.take<double>(3 * (size_t)n_ref_segments);
+  double* seg_inv = cv.take<double>(3 * (size_t)n_ref_segments);
   double* refs_sorted = cv.take<double>((size_t)n_refs * dim);
   int* ref_orig = cv.take<int>((size_t)n_refs);
   int* q_orig = cv.take<int>((size_t)n_queries);
@@ -380,19 +395,28 @@ int launch_knn_pruned(const double* refs, int ld_refs, const int* ref_off, const
     set_error("knn: workspace too small (%zu < %zu)", workspace_bytes, cv.used);
     return FB_ERR_WORKSPACE;
   }
-  k_pk_bbox<<<n_segments, 256, 0, stream>>>(refs, ld_refs, ref_off, queries, ld_queries, query_off, dim, seg_lo, seg_inv);
+  k_pk_bbox<<<n_ref_segments, 256, 0, stream>>>(refs, ld_refs, ref_off, queries, ld_queries, ref_seg ? nullptr : query_off,
+                                                dim, seg_lo, seg_inv);
   const int p2 = next_pow2(max_refs > max_queries ? max_refs : max_queries);
   const size_t sort_smem = sizeof(unsigned long long) * (size_t)p2;
   // the opt-in is per device and per function: set whenever it is needed (cheap), never cached process-wide
   if (sort_smem > 48 * 1024) FB_CUDA(cudaFuncSetAttribute(k_pk_sort, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sort_smem));
-  k_pk_sort<<<dim3(n_segments, 2), 1024, sort_smem, stream>>>(refs, ld_refs, ref_off, queries, ld_queries, query_off,
-                                                              dim, seg_lo, seg_inv, p2, refs_sorted, ref_orig, q_orig,
-                                                              q_key, tile_lo, tile_hi, tile_key);
+  k_pk_sort<<<dim3(n_ref_segments > n_segments ? n_ref_segments : n_segments, 2), 1024, sort_smem, stream>>>(
+      refs, ld_refs, ref_off, n_ref_segments, queries, ld_queries, query_off, n_segments, ref_seg, dim, seg_lo, seg_inv,
+      p2, refs_sorted, ref_orig, q_orig, q_key, tile_lo, tile_hi, tile_key);
   dim3 grid(div_up(max_queries, PK_TQ), n_segments);
   const size_t smem = sizeof(double) * PK_TR * dim + sizeof(int) * PK_TR;
-#define FB_PK(DD, KK)                                                                                              \
-  k_pk_search<DD, KK><<<grid, PK_TQ, smem, stream>>>(refs_sorted, ref_orig, ref_off, queries, ld_queries, query_off, \
-                                                     q_orig, q_key, tile_lo, tile_hi, tile_key, dim, k, idx, dist)
+#define FB_PK(DD, KK)                                                                                               \
+  do {                                                                                                              \
+    if (ref_seg)                                                                                                    \
+      k_pk_search<DD, KK, true><<<grid, PK_TQ, smem, stream>>>(refs_sorted, ref_orig, ref_off, ref_seg, queries,      \
+                                                               ld_queries, query_off, q_orig, q_key, tile_lo, tile_hi, \
+                                                               tile_key, dim, k, idx, dist);                          \
+    else                                                                                                            \
+      k_pk_search<DD, KK, false><<<grid, PK_TQ, smem, stream>>>(refs_sorted, ref_orig, ref_off, nullptr, queries,    \
+                                                                ld_queries, query_off, q_orig, q_key, tile_lo,        \
+                                                                tile_hi, tile_key, dim, k, idx, dist);                \
+  } while (0)
   if (dim == 3 && k == 1)
     FB_PK(3, 1);
   else if (dim == 3 && k == 3)
