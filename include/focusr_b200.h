@@ -77,6 +77,24 @@ int focusr_mean_filter(const int* row_ptr, const int* cols, const double* weight
                        double* values_out, int n_cols, int iterations, void* workspace,
                        size_t workspace_bytes, focusr_stream_t stream);
 
+/* K5 on mapped segments (a mesh smoothing several signals, as a source shared by several pairs): segment s smooths
+ * graph mesh seg_mesh[s] (device int32 [n_segments]; `seg_mesh_host` is its host copy, checked to lie in
+ * [0, n_meshes); `mesh_off_host` is the host copy of the graph's mesh offsets `mesh_off`).  The rows of segment s in
+ * values_in / values_out follow those of segments 0..s-1, each as many as its mesh has: row r of segment s (first
+ * value row seg0) is graph row mesh_off[m] + (r - seg0), and its neighbour j reads value row seg0 + (j - mesh_off[m]).
+ * A mesh may be mapped by several segments, by none, in any order.  The per-row arithmetic is that of
+ * focusr_mean_filter, so the result is bit-identical to focusr_mean_filter on a batch holding a copy of mesh seg_mesh[s]
+ * for every segment.  iterations == 0 copies values_in.  The launch table (one entry per CTA, no CTA spans two
+ * segments) is built from the host copies and staged through the workspace, which also holds the two ping-pong
+ * iterates.  Segments that are consecutive meshes in ascending order are smoothed by focusr_mean_filter's own kernel
+ * form, without the table. */
+size_t focusr_mean_filter_mapped_workspace_bytes(int n_rows, int n_cols, int n_segments);
+int focusr_mean_filter_mapped(const int* row_ptr, const int* cols, const double* weights, const double* degree,
+                              const int* mesh_off, const int* mesh_off_host, int n_meshes,
+                              const int* seg_mesh, const int* seg_mesh_host, int n_segments,
+                              const double* values_in, double* values_out, int n_cols, int iterations,
+                              void* workspace, size_t workspace_bytes, focusr_stream_t stream);
+
 /* out[i][:] = in[idx[i]][:]  (focusr.py:387 `smoothed_target_coords[corresponding_idx, :]`;
  * focusr.py:429-431 nearest-neighbour positions).  `idx_base[i]` (nullable) is added to idx[i]. */
 int focusr_gather_rows(const double* in, const long long* idx, const int* idx_base, int n_rows,

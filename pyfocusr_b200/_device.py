@@ -228,6 +228,29 @@ class DeviceGraph:
                   c, int(iterations), _lib.ptr(ws), ws_bytes, _lib.stream_ptr())
         return out
 
+    def mean_filter_mapped(self, values, iterations, seg_mesh):
+        """``focusr_mean_filter_mapped``: segment s of ``values`` (device [rows][c]; the segments' rows one after the
+        other, each as many as its mesh has) is smoothed on graph mesh ``seg_mesh[s]`` (host ints).  A mesh may serve
+        several segments or none.  Returns a new tensor, equal to :meth:`mean_filter` on a batch holding a copy of mesh
+        ``seg_mesh[s]`` for every segment."""
+        torch = _torch()
+        lib = _lib.load()
+        seg_host = np.ascontiguousarray(seg_mesh, dtype=np.int32).reshape(-1)
+        if seg_host.size and 0 <= seg_host.min() and seg_host.max() < self.n_meshes:  # otherwise the library says which
+            n_rows = int(np.diff(self.mesh_off_host.astype(np.int64))[seg_host].sum())
+            if int(values.shape[0]) != n_rows:
+                raise ValueError("mean_filter_mapped: the segments hold %d rows, values has %d" % (n_rows, values.shape[0]))
+        c = int(values.shape[1])
+        out = torch.empty_like(values)
+        ws_bytes = int(lib.focusr_mean_filter_mapped_workspace_bytes(int(values.shape[0]), c, int(seg_host.size)))
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=self.device)
+        seg_dev = torch.from_numpy(seg_host).to(self.device, non_blocking=True)
+        _lib.call("focusr_mean_filter_mapped", _lib.ptr(self.row_ptr), _lib.ptr(self.cols), _lib.ptr(self.weights),
+                  _lib.ptr(self.degree), _lib.ptr(self.mesh_off), _lib.ptr(self.mesh_off_host), self.n_meshes,
+                  _lib.ptr(seg_dev), _lib.ptr(seg_host), int(seg_host.size), _lib.ptr(values), _lib.ptr(out), c,
+                  int(iterations), _lib.ptr(ws), ws_bytes, _lib.stream_ptr())
+        return out
+
 
 # ---------------------------------------------------------------------------------------------
 # free functions on device tensors

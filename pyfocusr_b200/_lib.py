@@ -30,6 +30,8 @@ SIGNATURES = {
     "focusr_laplacian_csr": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
     "focusr_mean_filter_workspace_bytes": (_sz, [_i, _i]),
     "focusr_mean_filter": (_i, [_vp, _vp, _vp, _vp, _i, _i, _vp, _vp, _i, _i, _vp, _sz, _vp]),
+    "focusr_mean_filter_mapped_workspace_bytes": (_sz, [_i, _i, _i]),
+    "focusr_mean_filter_mapped": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _i, _vp, _vp, _i, _i, _vp, _sz, _vp]),
     "focusr_gather_rows": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp]),
     "focusr_eigs_workspace_bytes": (_sz, [_i, _i, _i, _i]),
     "focusr_sell_entries_cap": (C.c_longlong, [_vp, _vp, _i]),

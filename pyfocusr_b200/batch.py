@@ -12,7 +12,11 @@ of the vertices and the download of the correspondences except the eigensolver's
 Mesh order inside the batch graph: targets 0..P-1, then sources 0..P-1.  With ``run(..., target_of_pair=...)`` (many
 sources against a few templates) the batch graph holds T distinct targets, then the P sources, and pair p is target
 ``target_of_pair[p]`` with source p: each target is built, solved and smoothed once, and the results are returned in the
-pair layout (target copy p, then source p) of the batch with every target repeated once per pair.
+pair layout (target copy p, then source p) of the batch with every target repeated once per pair.  With
+``run(..., mesh_pairs=...)`` (all-vs-all, one subject against several atlases, both directions of a pair) the batch graph
+holds M meshes in any order and pair p is mesh ``mesh_pairs[p][0]`` with mesh ``mesh_pairs[p][1]``: each mesh is built
+and solved once, each target smoothed once, and every pair's projection smoothed on the one copy of its source's graph
+(``focusr_mean_filter_mapped``).  ``target_of_pair`` runs as ``mesh_pairs = [(target_of_pair[p], T + p)]``.
 """
 from __future__ import annotations
 
@@ -56,35 +60,80 @@ def shared_targets(target_of_pair, n_meshes, n_pairs):
     return top.astype(np.int32), T
 
 
+def mesh_pairs_checked(mesh_pairs, n_meshes, n_pairs=None):
+    """Checks ``mesh_pairs`` ((target mesh, source mesh) per pair) of a batch of ``n_meshes`` meshes and returns it as
+    int32 [P][2].  ``ValueError`` unless it is [P][2] with P >= 1 (and P == ``n_pairs`` when given), every value is an
+    integer in [0, n_meshes) and every mesh is used by some pair."""
+    mp = np.asarray(mesh_pairs)
+    if mp.ndim != 2 or mp.shape[1] != 2:
+        raise ValueError("mesh_pairs must be [P][2] (target mesh, source mesh), got shape %s" % (mp.shape,))
+    P, M = mp.shape[0], int(n_meshes)
+    if P < 1:
+        raise ValueError("mesh_pairs needs at least one pair")
+    if n_pairs is not None and int(n_pairs) != P:
+        raise ValueError("n_pairs (%d) must equal the number of mesh_pairs (%d)" % (int(n_pairs), P))
+    if mp.dtype.kind not in "iu":
+        if mp.dtype.kind != "f" or not np.all(np.isfinite(mp)) or not np.all(mp == np.round(mp)):
+            raise ValueError("mesh_pairs must hold integers")
+    mp = mp.astype(np.int64)
+    bad = np.argwhere((mp < 0) | (mp >= M))
+    if bad.size:
+        p, c = bad[0]
+        raise ValueError("mesh_pairs[%d][%d] = %d lies outside [0, %d)" % (p, c, mp[p, c], M))
+    unused = np.setdiff1d(np.arange(M), mp)
+    if unused.size:
+        raise ValueError("mesh(es) %s are used by no pair: a batch holds only the meshes its pairs use" % unused[:16].tolist())
+    return mp.astype(np.int32)
+
+
+def check_icp_moving(mesh_pairs, target_to_source):
+    """ICP moves one mesh of every pair, and the batch graph is built from the moved points: ``ValueError`` unless every
+    moving mesh is in exactly one pair and is not that pair's fixed mesh."""
+    fixed, moving = (mesh_pairs[:, 1], mesh_pairs[:, 0]) if target_to_source else (mesh_pairs[:, 0], mesh_pairs[:, 1])
+    for p, m in enumerate(moving):
+        pairs = np.nonzero((mesh_pairs == m).any(axis=1))[0]
+        if pairs.size != 1 or fixed[p] == m:
+            raise ValueError("ICP moves mesh %d (the %s of pair %d) onto mesh %d, but mesh %d is in pairs %s: a moving mesh "
+                             "must be in exactly one pair and not be that pair's fixed mesh" % (
+                                 m, "target" if target_to_source else "source", p, fixed[p], m, pairs.tolist()))
+
+
+def layout_rows(src_off, mesh_of, dev):
+    """A layout holding a copy of mesh ``mesh_of[i]`` of a batch with mesh offsets ``src_off`` (host), one after the
+    other: its mesh offsets (host int32) and the batch row of every one of its rows (device int64)."""
+    torch = _lib.require_cuda()
+    src_off = np.asarray(src_off, dtype=np.int64)
+    sizes = np.diff(src_off)[mesh_of]
+    off = np.zeros(sizes.size + 1, dtype=np.int32)
+    off[1:] = np.cumsum(sizes)
+    # each mesh's shift, repeated over the mesh's rows, plus the row itself
+    shift = torch.from_numpy(src_off[mesh_of] - off[:-1]).to(dev, non_blocking=True)
+    row_map = torch.arange(int(off[-1]), dtype=torch.int64, device=dev) + torch.repeat_interleave(
+        shift, torch.from_numpy(sizes).to(dev, non_blocking=True), output_size=int(off[-1]))
+    return off, row_map
+
+
 class PairLayout:
-    """The pair layout of a shared-target batch: 2P meshes, copy p of target ``target_of_pair[p]``, then source p.  It
-    stands in for the batch's ``DeviceGraph`` in the stages that work pair by pair (eigsort, spectral and feature
-    coordinates, CPD, the first KNN): same attributes (``mesh_off`` / ``mesh_off_host``, ``n_meshes``, ``n_points``,
-    ``max_mesh_points``, ``points``, ``device``) and the same column methods, but no Laplacian of its own.  ``rows``
-    gathers per-vertex rows of the batch graph into this layout (``focusr_gather_rows``)."""
+    """A layout of copies of batch meshes: mesh i is a copy of batch mesh ``mesh_of[i]``.  As the pair layout of a batch
+    with shared meshes (``mesh_of`` = the P targets, then the P sources of the pairs) it stands in for the batch's
+    ``DeviceGraph`` in the stages that work pair by pair (eigsort, spectral and feature coordinates, CPD, the first
+    KNN): same attributes (``mesh_off`` / ``mesh_off_host``, ``n_meshes``, ``n_points``, ``max_mesh_points``,
+    ``points``, ``device``) and the same column methods, but no Laplacian of its own.  ``rows`` gathers per-vertex rows
+    of the batch graph into this layout (``focusr_gather_rows``)."""
 
     flip_permute = DeviceGraph.flip_permute
     spectral_coords = DeviceGraph.spectral_coords
 
-    def __init__(self, g, target_of_pair):
+    def __init__(self, g, mesh_of):
         torch = _lib.require_cuda()
-        P = int(target_of_pair.size)
-        T = g.n_meshes - P
-        real_off = g.mesh_off_host.astype(np.int64)
-        self.mesh_of = np.concatenate([target_of_pair, np.arange(T, T + P)]).astype(np.int64)  # batch mesh of each mesh
-        sizes = np.diff(real_off)[self.mesh_of]
-        self.mesh_off_host = np.zeros(2 * P + 1, dtype=np.int32)
-        self.mesh_off_host[1:] = np.cumsum(sizes)
-        self.n_meshes = 2 * P
-        self.n_points = int(self.mesh_off_host[-1])
-        self.max_mesh_points = int(sizes.max())
+        self.mesh_of = np.asarray(mesh_of, dtype=np.int64)
         self.device = dev = g.device
+        self.mesh_off_host, self.row_map = layout_rows(g.mesh_off_host, self.mesh_of, dev)
+        self.n_meshes = int(self.mesh_of.size)
+        self.n_points = int(self.mesh_off_host[-1])
+        self.max_mesh_points = int(np.diff(self.mesh_off_host).max())
         self.mesh_off = torch.from_numpy(self.mesh_off_host).to(dev, non_blocking=True)
         self.mesh_map = torch.from_numpy(self.mesh_of).to(dev, non_blocking=True)
-        # batch row of every row of this layout: its mesh's shift, repeated over the mesh's rows, plus the row itself
-        shift = torch.from_numpy(real_off[self.mesh_of] - self.mesh_off_host[:-1]).to(dev, non_blocking=True)
-        self.row_map = torch.arange(self.n_points, dtype=torch.int64, device=dev) + torch.repeat_interleave(
-            shift, torch.from_numpy(sizes).to(dev, non_blocking=True), output_size=self.n_points)
         self.points = self.rows(g.points)
 
     def rows(self, values, n_rows=None):
@@ -207,7 +256,7 @@ class SpectralBatch:
 
     # ------------------------------------------------------------------------------------------
     def run(self, points, tris, mesh_off_host, n_pairs, idx_t=None, idx_s=None, record_events=False,
-            keep_presort=False, tri_off_host=None, node_features=None, target_of_pair=None):
+            keep_presort=False, tri_off_host=None, node_features=None, target_of_pair=None, mesh_pairs=None):
         """points: torch tensor [n_points_total, 3] float64 (host pinned or device), meshes in the
         order targets then sources; tris: int32 [n_tris_total, 3] with GLOBAL vertex ids;
         mesh_off_host: int32 [2P+1].  Returns a dict of device tensors + host metadata.
@@ -230,14 +279,31 @@ class SpectralBatch:
         batch with each target repeated once per pair, except ``graph`` and ``eigs_info``, which describe the T + P meshes
         built and solved.  ``pair_mesh_off`` holds the pair layout's mesh offsets (with ``target_of_pair=None``: those of
         ``graph``).  ``node_features`` and ``tri_off_host`` follow the T + P layout.  ``ValueError`` for a target outside
-        [0, T), a target no pair uses, or ``icp_reg_target_to_source`` with ICP on and a target shared by two pairs."""
+        [0, T), a target no pair uses, or ``icp_reg_target_to_source`` with ICP on and a target shared by two pairs.
+
+        ``mesh_pairs`` (int [P][2]): any (target mesh, source mesh) pairs over the M meshes of ``mesh_off_host``, in any
+        order; a mesh may be the target of some pairs and the source of others, in any number of pairs, and ``(m, m)``
+        is a pair.  Each mesh's Laplacian, eigenpairs and features are computed once, each target's 300 smoothing passes
+        once, and each pair's 40 projection passes run on the one copy of its source's graph.  Every key equals, bit for
+        bit, that of ``run`` on the pair layout (``run_meshes([meshes[t] for t, _ in mesh_pairs], [meshes[s] for _, s
+        in mesh_pairs])``), except ``graph`` and ``eigs_info``, which describe the M meshes; ``pair_mesh_off`` holds the
+        pair layout's offsets.  ``ValueError`` for a malformed list, a mesh outside [0, M) or used by no pair, ``n_pairs
+        != P``, ``target_of_pair`` given too, or, with ICP on, a moving mesh that is not in exactly one pair or is that
+        pair's fixed mesh.  ``target_of_pair`` is the case ``mesh_pairs = [(target_of_pair[p], T + p)]``."""
         P = int(n_pairs)
-        top = None
+        mp = None  # (target mesh, source mesh) of every pair when meshes are shared, else None (mesh p with mesh P + p)
+        if target_of_pair is not None and mesh_pairs is not None:
+            raise ValueError("give mesh_pairs or target_of_pair, not both (target_of_pair is mesh_pairs [(t, T + p)])")
         if target_of_pair is not None:
             top, T = shared_targets(target_of_pair, np.asarray(mesh_off_host).size - 1, P)
             if self.icp_register_first and self.icp_reg_target_to_source and np.unique(top).size < P:
                 raise ValueError("icp_reg_target_to_source moves each pair's target onto its source: a target shared by "
                                  "several pairs would move differently for each of them")
+            mp = np.stack([top, np.arange(T, T + P, dtype=np.int32)], axis=1)
+        elif mesh_pairs is not None:
+            mp = mesh_pairs_checked(mesh_pairs, np.asarray(mesh_off_host).size - 1, P)
+        if mp is not None and self.icp_register_first:
+            check_icp_moving(mp, self.icp_reg_target_to_source)
         n_mesh_feats = len(self.list_features_to_get_from_mesh)
         if n_mesh_feats:
             n_total = int(np.asarray(mesh_off_host)[-1])
@@ -258,7 +324,7 @@ class SpectralBatch:
         mark("start")
         icp_mats = None
         if self.icp_register_first:
-            points, tris, icp_mats = self._icp(points, tris, mesh_off_host, P, tri_off_host, top)
+            points, tris, icp_mats = self._icp(points, tris, mesh_off_host, P, tri_off_host, mp)
             mark("icp")
         feats, edge_points = None, None
         if self.features_on:
@@ -267,8 +333,21 @@ class SpectralBatch:
         g = DeviceGraph.from_device(points, tris, mesh_off_host, edge_points)
         mark("laplacian")
         n, ns = self.n, self.ns
-        nt_mesh = P if top is None else T  # targets in the batch graph
-        nt_total = int(g.mesh_off_host[nt_mesh])
+        if mp is None:
+            nt_total = int(g.mesh_off_host[P])
+
+            def smooth_targets():
+                return g.mean_filter(g.points, self.graph_smoothing_iterations, 0, nt_total)
+        else:  # the compact target block: the distinct targets in mesh order, cb_of[p] = pair p's target in it.  Mesh order
+            # makes the block the contiguous graph rows of consecutive targets (target_of_pair, all-vs-all), which
+            # focusr_mean_filter_mapped smooths with the identity form
+            tb = PairLayout(g, np.unique(mp[:, 0]))
+            cb_index = np.zeros(g.n_meshes, dtype=np.int32)
+            cb_index[tb.mesh_of] = np.arange(tb.n_meshes)
+            cb_of = cb_index[mp[:, 0]]
+
+            def smooth_targets():
+                return g.mean_filter_mapped(tb.points, self.graph_smoothing_iterations, tb.mesh_of)
         smoothed_t, side = None, None
         if self.overlap_smoothing:
             main = torch.cuda.current_stream()
@@ -277,7 +356,7 @@ class SpectralBatch:
             side = self._tls.side_stream
             side.wait_stream(main)
             with torch.cuda.stream(side):
-                smoothed_t = g.mean_filter(g.points, self.graph_smoothing_iterations, 0, nt_total)
+                smoothed_t = smooth_targets()
             smoothed_t.record_stream(main)
         try:
             vals, vecs, info = g.eigs_smallest(k=n + 1, n_k_needed=n, k_buffer=1, tol=self.tol,
@@ -287,27 +366,27 @@ class SpectralBatch:
             if info is None:
                 raise
             bad = np.nonzero(info["status"] != 0)[0]
-            if top is None:
+            if mp is None:
                 raise RuntimeError("eigensolve failed for %d of %d meshes: %s (mesh m is the %s of pair m %% %d); the other "
                                    "meshes of the batch were solved -- drop the named pairs and rerun" % (
                                        bad.size, 2 * P, ", ".join("mesh %d: %s" % (m, _device.EIG_STATUS.get(int(info["status"][m]), "?"))
                                                                   for m in bad[:16]), "target if m < %d else source" % P, P)) from exc
             raise RuntimeError("eigensolve failed for %d of %d meshes: %s; the other meshes of the batch were solved -- drop "
-                               "the named pairs and rerun" % (bad.size, T + P, ", ".join(
-                                   "%s: %s" % (self._mesh_pairs(m, top), _device.EIG_STATUS.get(int(info["status"][m]), "?"))
+                               "the named pairs and rerun" % (bad.size, g.n_meshes, ", ".join(
+                                   "%s: %s" % (self._mesh_pairs(m, mp), _device.EIG_STATUS.get(int(info["status"][m]), "?"))
                                    for m in bad[:16]))) from exc
         n_found = info["n_found"]
         if int(n_found.min()) < n:
             short = np.nonzero(n_found < n)[0]
-            if top is None:
+            if mp is None:
                 raise RuntimeError("meshes %s returned fewer than %d eigenpairs (pairs %s)" % (
                     short[:16].tolist(), n, sorted(set(int(m) % P for m in short[:16]))))
-            raise RuntimeError("fewer than %d eigenpairs for %s" % (n, "; ".join(self._mesh_pairs(m, top) for m in short[:16])))
+            raise RuntimeError("fewer than %d eigenpairs for %s" % (n, "; ".join(self._mesh_pairs(m, mp) for m in short[:16])))
         g.normalize_columns(vecs, n_found)
         mark("eigensolve")
         pg = g  # the graph of the pair stages: the batch graph itself, or its pair layout
-        if top is not None:  # gather the target rows into the pair layout; the sources keep their rows
-            pg = PairLayout(g, top)
+        if mp is not None:  # gather the rows of every pair's target, then of every pair's source, into the pair layout
+            pg = PairLayout(g, np.concatenate([mp[:, 0], mp[:, 1]]))
             vecs, vals, n_found = pg.rows(vecs), pg.meshes(vals), n_found[pg.mesh_of]
             mark("pair_layout")
 
@@ -335,7 +414,7 @@ class SpectralBatch:
                 parts = [g.mean_filter(feats[:, a:a + 8].contiguous(), self.feature_smoothing_iterations)
                          for a in range(0, self.n_node_features, 8)]
                 smoothed_f = parts[0] if len(parts) == 1 else torch.cat(parts, dim=1)
-                if top is not None:
+                if mp is not None:
                     smoothed_f = pg.rows(smoothed_f)
             coords = _device.feature_coords(coords, smoothed_f, pg.points, pg.mesh_off, self.include_points_as_features,
                                             self.norm_physical_and_spectral)
@@ -357,53 +436,57 @@ class SpectralBatch:
         if side is not None:
             torch.cuda.current_stream().wait_stream(side)
         else:
-            smoothed_t = g.mean_filter(g.points, self.graph_smoothing_iterations, 0, nt_total)
-        if top is None:
+            smoothed_t = smooth_targets()
+        if mp is None:
             base_q = torch.repeat_interleave(g.mesh_off[:P], torch.from_numpy(sizes[P:].astype(np.int64)).to(dev)).to(torch.int32)
-        else:  # the first row of each pair's target in the batch graph
-            base_q = torch.repeat_interleave(torch.from_numpy(g.mesh_off_host[top]).to(dev, non_blocking=True),
-                                             torch.from_numpy(sizes[P:].astype(np.int64)).to(dev, non_blocking=True),
-                                             output_size=g.n_points - nt_total)
-        staged = torch.empty_like(g.points)
-        _lib.call("focusr_gather_rows", _lib.ptr(smoothed_t), _lib.ptr(idx0), _lib.ptr(base_q), g.n_points - nt_total, 3,
-                  _lib.ptr(staged[nt_total:]), _lib.stream_ptr())
-        src_proj = g.mean_filter(staged, self.projection_smooth_iterations, nt_total, g.n_points)
+            staged = torch.empty_like(g.points)
+            _lib.call("focusr_gather_rows", _lib.ptr(smoothed_t), _lib.ptr(idx0), _lib.ptr(base_q), g.n_points - nt_total, 3,
+                      _lib.ptr(staged[nt_total:]), _lib.stream_ptr())
+            src_proj = g.mean_filter(staged, self.projection_smooth_iterations, nt_total, g.n_points)[nt_total:]
+        else:  # every pair's smoothed target, at idx0, smoothed on the one copy of its source's graph
+            q_sizes = torch.from_numpy(sizes[P:].astype(np.int64)).to(dev, non_blocking=True)
+            staged = _device.gather_rows(smoothed_t, idx0, torch.repeat_interleave(
+                torch.from_numpy(tb.mesh_off_host[cb_of]).to(dev, non_blocking=True), q_sizes, output_size=pg.n_points - nt_pair))
+            src_proj = g.mean_filter_mapped(staged, self.projection_smooth_iterations, mp[:, 1])
         mark("smoothing")
         # one k=3 search serves both focusr.py:391-392 (k=1: its first column, same distances and tie
         # rule) and focusr.py:409-413 (k=3)
-        if top is None:
-            idx3, dist3 = _device.knn(smoothed_t[:nt_total], src_proj[nt_total:], k=3, ref_off=ref_off, query_off=qry_off,
+        if mp is None:
+            idx3, dist3 = _device.knn(smoothed_t[:nt_total], src_proj, k=3, ref_off=ref_off, query_off=qry_off,
                                       max_queries=max_q, max_refs=max_r)
         else:  # each target's Morton sort and tiles serve all of its pairs
-            idx3, dist3 = _device.knn_mapped(smoothed_t[:nt_total], src_proj[nt_total:], g.mesh_off[: T + 1].contiguous(),
-                                             (g.mesh_off[T:] - nt_total).contiguous(), top, k=3, max_queries=max_q,
-                                             max_refs=int(np.diff(g.mesh_off_host[: T + 1]).max()))
+            idx3, dist3 = _device.knn_mapped(smoothed_t, src_proj, tb.mesh_off, qry_off, cb_of, k=3, max_queries=max_q,
+                                             max_refs=tb.max_mesh_points)
+            # the first row of each pair's target in the batch graph
+            base_q = torch.repeat_interleave(torch.from_numpy(g.mesh_off_host[mp[:, 0]]).to(dev, non_blocking=True),
+                                             q_sizes, output_size=pg.n_points - nt_pair)
         idx1 = idx3[:, :1]
         weighted = _device.weighted_positions(idx3, dist3, g.points, base_q)
         nearest = _device.gather_rows(g.points, idx1[:, 0].contiguous(), base_q)
         mark("knn_final")
-        smoothed_tc = smoothed_t[:nt_total] if top is None else pg.rows(smoothed_t, nt_pair)
-        if top is not None and feats is not None:
-            feats = pg.rows(feats)
+        if mp is None:
+            smoothed_tc = smoothed_t[:nt_total]
+        else:
+            smoothed_tc = _device.gather_rows(smoothed_t, layout_rows(tb.mesh_off_host, cb_of, dev)[1])
+            if feats is not None:
+                feats = pg.rows(feats)
         if record_events:
             torch.cuda.synchronize()
             self.timings = {ev[i][0]: ev[i - 1][1].elapsed_time(ev[i][1]) for i in range(1, len(ev))}
         return dict(graph=g, eig_vals=vals, eig_vecs=vecs, eigs_info=info, Q=Q, spectral_weights=weights[:P],
                     eigsort_status=decide_status, pair_mesh_off=off,
                     coords=coords, initial_idx=idx0[:, 0], smoothed_target_coords=smoothed_tc,
-                    source_projected_on_target=src_proj[nt_total:], final_idx=idx1[:, 0], knn3_idx=idx3,
+                    source_projected_on_target=src_proj, final_idx=idx1[:, 0], knn3_idx=idx3,
                     knn3_dist=dist3, weighted_avg_transformed_points=weighted,
                     nearest_neighbor_transformed_points=nearest, idx_t=idx_t, idx_s=idx_s, costs=costs,
                     eig_vecs_presort=presort, cpd_idx=cpd_idx, coords_b4_reg=coords_b4_reg, icp_matrices=icp_mats,
                     node_features=feats)
 
     @staticmethod
-    def _mesh_pairs(m, top):
-        """Mesh m of a shared-target batch graph named by the pairs it serves."""
-        T = int(top.max()) + 1
-        if m < T:
-            return "target %d (pairs %s)" % (m, np.nonzero(top == m)[0].tolist())
-        return "source of pair %d" % (m - T)
+    def _mesh_pairs(m, mesh_pairs):
+        """Mesh m of a batch graph with shared meshes named by every pair it serves."""
+        t, s = (np.nonzero(mesh_pairs[:, c] == m)[0].tolist() for c in (0, 1))
+        return "mesh %d (%s)" % (m, ", ".join((["target of pairs %s" % t] if t else []) + (["source of pairs %s" % s] if s else [])))
 
     def _node_features(self, points, tris, mesh_off_host, node_features):
         """graph.py:84-142,166-175 for every mesh at once: curvature of the (moved) points in one focusr_curvatures call
@@ -434,10 +517,10 @@ class SpectralBatch:
                                                    want_edge_points=self.features_in_adjacency)
         return pts, tr, feats, edge_points
 
-    def _icp(self, points, tris, mesh_off_host, P, tri_off_host, target_of_pair=None):
+    def _icp(self, points, tris, mesh_off_host, P, tri_off_host, mesh_pairs=None):
         """focusr.py:110-131 for every pair at once (``focusr_icp_batch``): returns the device points with each pair's
         moving mesh registered onto its fixed one (a new tensor), the device triangles and the (P, 4, 4) matrices.  With
-        ``target_of_pair`` pair p is batch mesh ``target_of_pair[p]`` with mesh T + p."""
+        ``mesh_pairs`` pair p is batch mesh ``mesh_pairs[p][0]`` with mesh ``mesh_pairs[p][1]``."""
         torch = _lib.require_cuda()
         off = np.ascontiguousarray(mesh_off_host, dtype=np.int32)
         if tri_off_host is None:
@@ -446,9 +529,8 @@ class SpectralBatch:
         pts = points.to(dev, non_blocking=True).contiguous()
         tr = tris.to(dev, non_blocking=True).contiguous()
         targets, sources = np.arange(P, dtype=np.int32), np.arange(P, 2 * P, dtype=np.int32)
-        if target_of_pair is not None:
-            T = off.size - 1 - P
-            targets, sources = np.asarray(target_of_pair, dtype=np.int32), np.arange(T, T + P, dtype=np.int32)
+        if mesh_pairs is not None:
+            targets, sources = mesh_pairs[:, 0].copy(), mesh_pairs[:, 1].copy()
         fixed, moving = (sources, targets) if self.icp_reg_target_to_source else (targets, sources)
         mats, moved = _device.icp_batch_device(pts, tr, off, tri_off_host, fixed, moving, max_iterations=100,
                                                max_landmarks=1000, similarity=self.icp_registration_mode == "similarity")
@@ -665,26 +747,45 @@ class SpectralBatch:
 
     # ------------------------------------------------------------------------------------------
     @staticmethod
-    def pack_meshes(targets, sources, target_of_pair=None):
-        """Lists of PolyData-like meshes (``.points``, ``.tris``) -> ``(points, tris, mesh_off_host, n_pairs)`` of ``run``
-        (host tensors; targets first, then sources; triangle vertex ids made global).  With ``target_of_pair`` (int [P],
-        one entry per source) the targets are the T shared ones, pair p being ``targets[target_of_pair[p]]`` with
-        ``sources[p]``; without it, pair p is ``targets[p]`` with ``sources[p]``."""
+    def _pack(meshes):
+        """A list of PolyData-like meshes (``.points``, ``.tris``) -> host ``(points, tris, mesh_off_host)``, the meshes
+        in list order, triangle vertex ids made global."""
         import torch
 
-        if target_of_pair is None:
-            if len(targets) != len(sources) or not targets:
-                raise ValueError("need as many source meshes as target meshes (at least one pair)")
-        else:
-            shared_targets(target_of_pair, len(targets) + len(sources), len(sources))
-        meshes = list(targets) + list(sources)
         sizes = [m.points.shape[0] for m in meshes]
         off = np.zeros(len(meshes) + 1, dtype=np.int32)
         off[1:] = np.cumsum(sizes)
         pts = torch.from_numpy(np.ascontiguousarray(np.concatenate([m.points for m in meshes])))
         tris = torch.from_numpy(np.ascontiguousarray(np.concatenate(
             [m.tris.astype(np.int64) + int(o) for m, o in zip(meshes, off[:-1])]).astype(np.int32)))
-        return pts, tris, off, len(sources)
+        return pts, tris, off
+
+    @staticmethod
+    def pack_meshes(targets, sources, target_of_pair=None):
+        """Lists of PolyData-like meshes (``.points``, ``.tris``) -> ``(points, tris, mesh_off_host, n_pairs)`` of ``run``
+        (host tensors; targets first, then sources; triangle vertex ids made global).  With ``target_of_pair`` (int [P],
+        one entry per source) the targets are the T shared ones, pair p being ``targets[target_of_pair[p]]`` with
+        ``sources[p]``; without it, pair p is ``targets[p]`` with ``sources[p]``."""
+        if target_of_pair is None:
+            if len(targets) != len(sources) or not targets:
+                raise ValueError("need as many source meshes as target meshes (at least one pair)")
+        else:
+            shared_targets(target_of_pair, len(targets) + len(sources), len(sources))
+        return SpectralBatch._pack(list(targets) + list(sources)) + (len(sources),)
+
+    def _run_packed(self, meshes, pts, tris, off, n_pairs, kw):
+        """``run`` on meshes packed by ``_pack``, with their point scalars (``list_features_to_get_from_mesh``) and
+        triangle ranges filled in unless given."""
+        if self.list_features_to_get_from_mesh and "node_features" not in kw:
+            import torch
+
+            kw["node_features"] = torch.from_numpy(np.ascontiguousarray(np.stack(
+                [np.concatenate([mesh_point_scalars(m, name).reshape(-1) for m in meshes])
+                 for name in self.list_features_to_get_from_mesh], axis=1)))
+        tri_off = np.zeros(len(meshes) + 1, dtype=np.int32)
+        tri_off[1:] = np.cumsum([m.tris.shape[0] for m in meshes])
+        kw.setdefault("tri_off_host", tri_off)
+        return self.run(pts, tris, off, n_pairs, **kw)
 
     def run_meshes(self, targets, sources, target_of_pair=None, **kw):
         """Convenience: lists of PolyData-like meshes (``.points``, ``.tris``); the point scalars named by
@@ -693,13 +794,13 @@ class SpectralBatch:
         pts, tris, off, n_pairs = self.pack_meshes(targets, sources, target_of_pair)
         if target_of_pair is not None:
             kw["target_of_pair"] = target_of_pair
-        if self.list_features_to_get_from_mesh and "node_features" not in kw:
-            import torch
+        return self._run_packed(list(targets) + list(sources), pts, tris, off, n_pairs, kw)
 
-            kw["node_features"] = torch.from_numpy(np.ascontiguousarray(np.stack(
-                [np.concatenate([mesh_point_scalars(m, name).reshape(-1) for m in list(targets) + list(sources)])
-                 for name in self.list_features_to_get_from_mesh], axis=1)))
-        tri_off = np.zeros(len(targets) + len(sources) + 1, dtype=np.int32)
-        tri_off[1:] = np.cumsum([m.tris.shape[0] for m in list(targets) + list(sources)])
-        kw.setdefault("tri_off_host", tri_off)
-        return self.run(pts, tris, off, n_pairs, **kw)
+    def run_mesh_pairs(self, meshes, mesh_pairs, **kw):
+        """Convenience for ``run(..., mesh_pairs=...)``: a list of M PolyData-like meshes, each packed once in list order,
+        and ``mesh_pairs`` [P][2] of (target, source) indices into it (all-vs-all, one subject against several atlases,
+        both directions of a pair...).  Point scalars and triangle ranges are filled in as by ``run_meshes``."""
+        meshes = list(meshes)
+        mp = mesh_pairs_checked(mesh_pairs, len(meshes))
+        pts, tris, off = self._pack(meshes)
+        return self._run_packed(meshes, pts, tris, off, mp.shape[0], dict(kw, mesh_pairs=mp))

@@ -31,6 +31,7 @@
 //     columns, weights and iterate rows of a row before its arithmetic (rows <= 8 entries; 80 registers, 3 CTAs per SM)
 //     was measured at 21.1 ms against 17.15 ms for the serial walk (gpurun_out/r2d_kernel_ab.log) and removed: fewer
 //     resident threads cost more than the longer load batches of each thread bring.
+#include <climits>
 #include <vector>
 
 #include "common.cuh"
@@ -942,21 +943,34 @@ int launch_filter_persist(bool corr, int b, const PersistArgs& a, cudaStream_t s
 #ifndef FB_SMOOTH_MINB
 #define FB_SMOOTH_MINB (2048 / FB_SMOOTH_THREADS)
 #endif
-template <int C>
+// MAP = false: value row = graph row, rows [row_begin, row_end) (focusr_mean_filter).  MAP = true: CTA b smooths graph
+// rows [t.x, t.x + t.y) with t = cta_rows[b], and graph row i is value row i + t.z (focusr_mean_filter_mapped).  The
+// host builds the table so that no CTA spans two segments: one table load per thread, no search, and the CTA's graph
+// rows stay contiguous, so the L2 prefetch of its matrix slice is that of the identity form.
+template <int C, bool MAP>
 __global__ void __launch_bounds__(FB_SMOOTH_THREADS, FB_SMOOTH_MINB)
 k_mean_filter(const int* __restrict__ row_ptr, const int* __restrict__ cols, const double* __restrict__ weights,
-              const double* __restrict__ degree, int row_begin, int row_end, const double* __restrict__ x,
-              double* __restrict__ out, int n_cols_rt) {
-  const int i = row_begin + blockIdx.x * blockDim.x + threadIdx.x;
+              const double* __restrict__ degree, int row_begin, int row_end, const int4* __restrict__ cta_rows,
+              const double* __restrict__ x, double* __restrict__ out, int n_cols_rt) {
+  int c0, c1, shift = 0;
+  if (MAP) {
+    const int4 t = cta_rows[blockIdx.x];
+    c0 = t.x;
+    c1 = t.x + t.y;
+    shift = t.z;
+  } else {
+    c0 = row_begin + blockIdx.x * blockDim.x;
+    c1 = min(row_end, c0 + (int)blockDim.x);
+  }
+  const int i = c0 + threadIdx.x;
   {
-    const int c0 = row_begin + blockIdx.x * blockDim.x, c1 = min(row_end, c0 + (int)blockDim.x);
     const int q0 = row_ptr[c0], q1 = row_ptr[c1];
     for (int q = q0 + 32 * (int)threadIdx.x; q < q1; q += 32 * (int)blockDim.x) prefetch_l2_line(cols + q);
     for (int q = q0 + 16 * (int)threadIdx.x; q < q1; q += 16 * (int)blockDim.x) prefetch_l2_line(weights + q);
   }
   pdl_wait();
   pdl_launch_dependents();
-  if (i >= row_end) return;
+  if (i >= (MAP ? c1 : row_end)) return;
   const int nc = C > 0 ? C : n_cols_rt;
   const double dsm = FB_DIV(1.0, FB_ADD(1.0, degree[i]));
   const int p0 = row_ptr[i], p1 = row_ptr[i + 1];
@@ -969,7 +983,7 @@ k_mean_filter(const int* __restrict__ row_ptr, const int* __restrict__ cols, con
     const int j = cols[p];
     const double wp = weights[p];
     if (!diag_done && j < i) {
-      const double* xi = x + (size_t)i * nc;
+      const double* xi = x + (size_t)(i + shift) * nc;
 #pragma unroll
       for (int k = 0; k < CMAX; ++k)
         if (k < nc) acc[k] = FB_ADD(acc[k], FB_MUL(dsm, xi[k]));
@@ -982,18 +996,18 @@ k_mean_filter(const int* __restrict__ row_ptr, const int* __restrict__ cols, con
     } else {
       val = FB_MUL(dsm, wp);
     }
-    const double* xj = x + (size_t)j * nc;
+    const double* xj = x + (size_t)(j + shift) * nc;
 #pragma unroll
     for (int k = 0; k < CMAX; ++k)
       if (k < nc) acc[k] = FB_ADD(acc[k], FB_MUL(val, xj[k]));
   }
   if (!diag_done) {
-    const double* xi = x + (size_t)i * nc;
+    const double* xi = x + (size_t)(i + shift) * nc;
 #pragma unroll
     for (int k = 0; k < CMAX; ++k)
       if (k < nc) acc[k] = FB_ADD(acc[k], FB_MUL(dsm, xi[k]));
   }
-  double* o = out + (size_t)i * nc;
+  double* o = out + (size_t)(i + shift) * nc;
 #pragma unroll
   for (int k = 0; k < CMAX; ++k)
     if (k < nc) o[k] = acc[k];
@@ -1016,6 +1030,47 @@ static SmoothLayout smooth_layout(int n_rows, int n_cols, void* ws) {
   l.buf_b = cv.take<double>((size_t)n_rows * n_cols);
   l.bytes = cv.used + 256;
   return l;
+}
+
+// the mapped form adds its CTA table: segment s of n_s rows takes ceil(n_s / threads) CTAs, so n_rows / threads +
+// n_segments entries bound it
+static SmoothLayout smooth_mapped_layout(int n_rows, int n_cols, int n_segments, void* ws, int4** table) {
+  Carver cv(ws, (size_t)-1);
+  SmoothLayout l;
+  l.buf_a = cv.take<double>((size_t)n_rows * n_cols);
+  l.buf_b = cv.take<double>((size_t)n_rows * n_cols);
+  *table = cv.take<int4>((size_t)n_rows / FB_SMOOTH_THREADS + n_segments + 1);
+  l.bytes = cv.used + 256;
+  return l;
+}
+
+// the chain of passes of both entry points: ping-pong between pa and pb, the last pass into out
+template <bool MAP>
+static int smooth_chain(const int* row_ptr, const int* cols, const double* weights, const double* degree, int row_begin,
+                        int row_end, const int4* cta_rows, int n_ctas, const double* src, double* pa, double* pb,
+                        double* out, int n_cols, int iterations, cudaStream_t stream) {
+  const dim3 grid(n_ctas), block(FB_SMOOTH_THREADS);
+  for (int it = 0; it < iterations; ++it) {
+    double* dst = it == iterations - 1 ? out : ((it & 1) ? pb : pa);
+    cudaError_t e;
+#define FB_SMOOTH(CC, NC)                                                                                             \
+  launch_pdl(k_mean_filter<CC, MAP>, grid, block, stream, row_ptr, cols, weights, degree, row_begin, row_end, cta_rows, \
+             src, dst, NC)
+    if (n_cols == 3)
+      e = FB_SMOOTH(3, 3);
+    else if (n_cols == 1)
+      e = FB_SMOOTH(1, 1);
+    else if (n_cols == 2)  // the two curvature columns of node features (SpectralBatch)
+      e = FB_SMOOTH(2, 2);
+    else
+      e = FB_SMOOTH(0, n_cols);
+#undef FB_SMOOTH
+    FB_CUDA(e);
+    src = dst;
+  }
+  FB_COUNT_LAUNCH(iterations);
+  FB_LAUNCH_CHECK();
+  return FB_OK;
 }
 
 }  // namespace fb
@@ -1050,26 +1105,68 @@ int focusr_mean_filter(const int* row_ptr, const int* cols, const double* weight
              "mean_filter: workspace too small (%zu < %zu)", workspace_bytes, l.bytes);
   // ping-pong between two buffers indexed by global row (shifted so that row_begin lands on their start)
   const size_t rb = (size_t)row_begin;
-  double* pa = l.buf_a - rb * n_cols;
-  double* pb = l.buf_b - rb * n_cols;
-  const double* src = values_in;
-  const dim3 grid(div_up(n, T)), block(T);
-  for (int it = 0; it < iterations; ++it) {
-    double* dst = it == iterations - 1 ? values_out : ((it & 1) ? pb : pa);
-    cudaError_t e;
-    if (n_cols == 3)
-      e = launch_pdl(k_mean_filter<3>, grid, block, stream, row_ptr, cols, weights, degree, row_begin, row_end, src, dst, 3);
-    else if (n_cols == 1)
-      e = launch_pdl(k_mean_filter<1>, grid, block, stream, row_ptr, cols, weights, degree, row_begin, row_end, src, dst, 1);
-    else if (n_cols == 2)  // the two curvature columns of node features (SpectralBatch)
-      e = launch_pdl(k_mean_filter<2>, grid, block, stream, row_ptr, cols, weights, degree, row_begin, row_end, src, dst, 2);
-    else
-      e = launch_pdl(k_mean_filter<0>, grid, block, stream, row_ptr, cols, weights, degree, row_begin, row_end, src, dst, n_cols);
-    FB_CUDA(e);
-    src = dst;
+  return smooth_chain<false>(row_ptr, cols, weights, degree, row_begin, row_end, nullptr, div_up(n, T), values_in,
+                             l.buf_a - rb * n_cols, l.buf_b - rb * n_cols, values_out, n_cols, iterations, stream);
+}
+
+size_t focusr_mean_filter_mapped_workspace_bytes(int n_rows, int n_cols, int n_segments) {
+  int4* table;
+  return smooth_mapped_layout(n_rows, n_cols, n_segments, nullptr, &table).bytes;
+}
+
+int focusr_mean_filter_mapped(const int* row_ptr, const int* cols, const double* weights, const double* degree,
+                              const int* mesh_off, const int* mesh_off_host, int n_meshes, const int* seg_mesh,
+                              const int* seg_mesh_host, int n_segments, const double* values_in, double* values_out,
+                              int n_cols, int iterations, void* workspace, size_t workspace_bytes,
+                              focusr_stream_t stream_) {
+  cudaStream_t stream = (cudaStream_t)stream_;
+  (void)mesh_off;
+  (void)seg_mesh;
+  FB_REQUIRE(n_meshes > 0 && n_segments > 0 && n_cols >= 1 && n_cols <= 8 && iterations >= 0,
+             "mean_filter_mapped: need meshes and segments, 1 <= n_cols <= 8, iterations >= 0");
+  FB_REQUIRE(mesh_off_host != nullptr && seg_mesh_host != nullptr,
+             "mean_filter_mapped: the host copies of mesh_off and seg_mesh are required");
+  long long n_rows = 0;
+  for (int s = 0; s < n_segments; ++s) {
+    const int m = seg_mesh_host[s];
+    FB_REQUIRE(m >= 0 && m < n_meshes, "mean_filter_mapped: segment %d maps to mesh %d, outside [0, %d)", s, m, n_meshes);
+    n_rows += mesh_off_host[m + 1] - mesh_off_host[m];
   }
-  FB_COUNT_LAUNCH(iterations);
-  FB_LAUNCH_CHECK();
-  return FB_OK;
+  FB_REQUIRE(n_rows > 0 && n_rows <= INT_MAX, "mean_filter_mapped: the segments hold %lld rows", n_rows);
+  const int T = FB_SMOOTH_THREADS;
+  if (iterations == 0) {
+    k_copy_rows<<<div_up(n_rows * n_cols, T), T, 0, stream>>>(values_in, values_out, 0, n_rows * n_cols);
+    FB_COUNT_LAUNCH(1);
+    FB_LAUNCH_CHECK();
+    return FB_OK;
+  }
+  int4* table;
+  const SmoothLayout l = smooth_mapped_layout((int)n_rows, n_cols, n_segments, workspace, &table);
+  FB_REQUIRE(workspace != nullptr && workspace_bytes >= l.bytes, "mean_filter_mapped: workspace too small (%zu < %zu)",
+             workspace_bytes, l.bytes);
+  // Segments that are consecutive graph meshes in ascending order are the graph rows [rb, re) shifted by rb: the
+  // identity form on pointers shifted by rb rows, as focusr_mean_filter shifts its ping-pong buffers.  The table form
+  // costs a dependent table load in every CTA's prologue (B200 at 1000 W, 128 meshes of 15 212 vertices: 18.1 against
+  // 17.2 ms for 300 passes, tools/batch_mesh_pairs_bench.py), so the identity form is used wherever the map allows it.
+  bool run = true;
+  for (int s = 1; s < n_segments && run; ++s) run = seg_mesh_host[s] == seg_mesh_host[s - 1] + 1;
+  if (run) {
+    const int rb = mesh_off_host[seg_mesh_host[0]], re = mesh_off_host[seg_mesh_host[n_segments - 1] + 1];
+    const size_t sh = (size_t)rb * n_cols;
+    return smooth_chain<false>(row_ptr, cols, weights, degree, rb, re, nullptr, div_up(re - rb, T), values_in - sh,
+                               l.buf_a - sh, l.buf_b - sh, values_out - sh, n_cols, iterations, stream);
+  }
+  // one entry per CTA {first graph row, rows, value row - graph row}; tiny, built here and staged by the runtime
+  // (pageable source)
+  std::vector<int4> cta;
+  int seg0 = 0;
+  for (int s = 0; s < n_segments; ++s) {
+    const int m = seg_mesh_host[s], g0 = mesh_off_host[m], n = mesh_off_host[m + 1] - g0;
+    for (int r = 0; r < n; r += T) cta.push_back(make_int4(g0 + r, n - r < T ? n - r : T, seg0 - g0, 0));
+    seg0 += n;
+  }
+  FB_CUDA(cudaMemcpyAsync(table, cta.data(), sizeof(int4) * cta.size(), cudaMemcpyHostToDevice, stream));
+  return smooth_chain<true>(row_ptr, cols, weights, degree, 0, 0, table, (int)cta.size(), values_in, l.buf_a, l.buf_b,
+                            values_out, n_cols, iterations, stream);
 }
 }
