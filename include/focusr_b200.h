@@ -252,9 +252,19 @@ int focusr_spectral_coords(const double* vecs, int n_points, int ld, const int* 
  * pairs.  Pair p uses mesh t_mesh[p] / s_mesh[p] of the batch, sample rows idx_t[p][0..n_samp_t)
  * and idx_s[p][..] (local row ids = Graph.rand_idxs).  Outputs [n_pairs][n][n] each:
  * c_hist / c_hist_f (1-D Wasserstein distance of log(v + 0.5 + eps), source flipped for _f) and
- * c_spatial / c_spatial_f (RMS difference at xyz nearest neighbours / n_samp_t); nn_idx
+ * c_spatial / c_spatial_f (RMS difference at xyz nearest neighbours / the pair's target samples); nn_idx
  * [n_pairs][n_samp_t] is the nearest sampled source point of each sampled target point.
  * c_lambda, min/compare, the n x n assignment and the flip list: focusr_eigsort_decide (device) or the host classes.
+ * Any number of samples: each column is sorted in one CTA's shared memory while the call's largest pair holds at most
+ * 16384 samples per mesh, else all columns go through one global segmented radix sort; both give the same sorted values,
+ * so the costs do not depend on which sort ran.  Does not synchronise.
+ *
+ * focusr_eigsort_costs_ragged: the same with a sample count per pair.  Pair p's target samples are
+ * idx_t[samp_off_t[p] .. samp_off_t[p+1]) and its source samples idx_s[samp_off_s[p] .. samp_off_s[p+1]) (offsets
+ * from 0, strictly increasing: no pair is empty); nn_idx [samp_off_t[n_pairs]] follows the target-sample layout, each
+ * index local to the pair's source samples.  The `_host` arrays are host copies of the device arrays of the same
+ * name (workspace size and launch sizing); the workspace size is 0 for an invalid description.  focusr_eigsort_costs
+ * is the case samp_off_t[p] = p * n_samp_t, samp_off_s[p] = p * n_samp_s, bit for bit.
  * ------------------------------------------------------------------------------------------- */
 size_t focusr_eigsort_workspace_bytes(int n_pairs, int n_samp_t, int n_samp_s, int n_features);
 int focusr_eigsort_costs(const double* vecs, int ld, const double* points,
@@ -263,6 +273,14 @@ int focusr_eigsort_costs(const double* vecs, int ld, const double* points,
                          int n_samp_s, int n_features, double* c_hist, double* c_hist_f,
                          double* c_spatial, double* c_spatial_f, long long* nn_idx, void* workspace,
                          size_t workspace_bytes, focusr_stream_t stream);
+size_t focusr_eigsort_ragged_workspace_bytes(const int* samp_off_t_host, const int* samp_off_s_host, int n_pairs,
+                                             int n_features);
+int focusr_eigsort_costs_ragged(const double* vecs, int ld, const double* points, const int* mesh_point_off,
+                                const int* t_mesh, const int* s_mesh, int n_pairs, const long long* idx_t,
+                                const long long* idx_s, const int* samp_off_t, const int* samp_off_s,
+                                const int* samp_off_t_host, const int* samp_off_s_host, int n_features, double* c_hist,
+                                double* c_hist_f, double* c_spatial, double* c_spatial_f, long long* nn_idx,
+                                void* workspace, size_t workspace_bytes, focusr_stream_t stream);
 
 /* C2, C5, D1  the n x n decisions of eigsort for every pair, on the device (eigsort.py:66-122, 142-160; focusr.py:
  * 459-490): c_lambda from the eigenvalues (`eig_vals` [n_meshes][ldv], `n_found` [n_meshes] = how many each mesh

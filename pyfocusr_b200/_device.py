@@ -535,27 +535,58 @@ def eigsort_decide(graph, vals, n_found, t_mesh, s_mesh, costs, n_features, ns, 
     return q, dst, src, sign, w, status
 
 
+def sample_rows(idx):
+    """Ordering samples of a batch, as ``eigsort_costs`` takes them: a 2-D [P][n] array (every pair the same count) stays
+    a 2-D int64 array; anything else is read as a sequence of P 1-D arrays (a count per pair) and returned as a list of
+    1-D int64 arrays."""
+    if getattr(idx, "ndim", None) == 2:
+        return np.ascontiguousarray(idx, dtype=np.int64)
+    return [np.asarray(r, dtype=np.int64).reshape(-1) for r in idx]
+
+
 def eigsort_costs(graph, vecs, t_mesh, s_mesh, idx_t, idx_s, n_features):
     """Cost matrices of eigsort for pairs (t_mesh[p], s_mesh[p]) of ``graph``.
-    idx_t / idx_s: host int arrays [n_pairs][n_samples] (Graph.rand_idxs).  Returns device tensors
-    (c_hist, c_hist_f, c_spatial, c_spatial_f) each [n_pairs][n][n] and nn_idx [n_pairs][n_samp_t]."""
+    idx_t / idx_s: host int arrays [n_pairs][n_samples] (Graph.rand_idxs), or sequences of n_pairs 1-D arrays (a sample
+    count per pair: ``focusr_eigsort_costs_ragged``).  Returns device tensors (c_hist, c_hist_f, c_spatial, c_spatial_f)
+    each [n_pairs][n][n] and nn_idx: [n_pairs][n_samp_t] for 2-D input, else a list of per-pair [n_t] views."""
     torch = _torch()
     lib = _lib.load()
     dev = graph.device
-    idx_t = np.ascontiguousarray(idx_t, dtype=np.int64)
-    idx_s = np.ascontiguousarray(idx_s, dtype=np.int64)
-    n_pairs, n_t = idx_t.shape
-    n_s = idx_s.shape[1]
+    idx_t, idx_s = sample_rows(idx_t), sample_rows(idx_s)
     n = int(n_features)
-    it = torch.from_numpy(idx_t).to(dev)
-    is_ = torch.from_numpy(idx_s).to(dev)
     tm, sm = _dev_i32(t_mesh), _dev_i32(s_mesh)
+    n_pairs = int(tm.shape[0])
     outs = [torch.empty((n_pairs, n, n), dtype=torch.float64, device=dev) for _ in range(4)]
-    nn = torch.empty((n_pairs, n_t), dtype=torch.int64, device=dev)
-    ws_bytes = int(lib.focusr_eigsort_workspace_bytes(n_pairs, n_t, n_s, n))
+    if isinstance(idx_t, np.ndarray) and isinstance(idx_s, np.ndarray):
+        n_t, n_s = idx_t.shape[1], idx_s.shape[1]
+        it = torch.from_numpy(idx_t).to(dev)
+        is_ = torch.from_numpy(idx_s).to(dev)
+        nn = torch.empty((n_pairs, n_t), dtype=torch.int64, device=dev)
+        ws_bytes = int(lib.focusr_eigsort_workspace_bytes(n_pairs, n_t, n_s, n))
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        _lib.call("focusr_eigsort_costs", _lib.ptr(vecs), int(vecs.shape[1]), _lib.ptr(graph.points), _lib.ptr(graph.mesh_off),
+                  _lib.ptr(tm), _lib.ptr(sm), n_pairs, _lib.ptr(it), _lib.ptr(is_), n_t, n_s, n, _lib.ptr(outs[0]),
+                  _lib.ptr(outs[1]), _lib.ptr(outs[2]), _lib.ptr(outs[3]), _lib.ptr(nn), _lib.ptr(ws), ws_bytes,
+                  _lib.stream_ptr())
+        return outs[0], outs[1], outs[2], outs[3], nn
+    rows_t, rows_s = list(idx_t), list(idx_s)
+    if len(rows_t) != n_pairs or len(rows_s) != n_pairs:
+        raise ValueError("eigsort_costs: %d pairs, but %d target and %d source sample arrays" % (n_pairs, len(rows_t), len(rows_s)))
+    cnt_t = np.array([r.size for r in rows_t], dtype=np.int64)
+    off_t = np.zeros(n_pairs + 1, dtype=np.int32)
+    off_t[1:] = np.cumsum(cnt_t)
+    off_s = np.zeros(n_pairs + 1, dtype=np.int32)
+    off_s[1:] = np.cumsum([r.size for r in rows_s])
+    it = torch.from_numpy(np.concatenate(rows_t)).to(dev)
+    is_ = torch.from_numpy(np.concatenate(rows_s)).to(dev)
+    ot, os_ = torch.from_numpy(off_t).to(dev), torch.from_numpy(off_s).to(dev)
+    nn = torch.empty(int(off_t[-1]), dtype=torch.int64, device=dev)
+    ws_bytes = int(lib.focusr_eigsort_ragged_workspace_bytes(_lib.ptr(off_t), _lib.ptr(off_s), n_pairs, n))
+    if ws_bytes == 0:
+        raise ValueError("eigsort_costs: every pair needs at least one target and one source sample")
     ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
-    _lib.call("focusr_eigsort_costs", _lib.ptr(vecs), int(vecs.shape[1]), _lib.ptr(graph.points), _lib.ptr(graph.mesh_off),
-              _lib.ptr(tm), _lib.ptr(sm), n_pairs, _lib.ptr(it), _lib.ptr(is_), n_t, n_s, n, _lib.ptr(outs[0]),
-              _lib.ptr(outs[1]), _lib.ptr(outs[2]), _lib.ptr(outs[3]), _lib.ptr(nn), _lib.ptr(ws), ws_bytes,
-              _lib.stream_ptr())
-    return outs[0], outs[1], outs[2], outs[3], nn
+    _lib.call("focusr_eigsort_costs_ragged", _lib.ptr(vecs), int(vecs.shape[1]), _lib.ptr(graph.points),
+              _lib.ptr(graph.mesh_off), _lib.ptr(tm), _lib.ptr(sm), n_pairs, _lib.ptr(it), _lib.ptr(is_), _lib.ptr(ot),
+              _lib.ptr(os_), _lib.ptr(off_t), _lib.ptr(off_s), n, _lib.ptr(outs[0]), _lib.ptr(outs[1]), _lib.ptr(outs[2]),
+              _lib.ptr(outs[3]), _lib.ptr(nn), _lib.ptr(ws), ws_bytes, _lib.stream_ptr())
+    return outs[0], outs[1], outs[2], outs[3], list(torch.split(nn, cnt_t.tolist()))

@@ -61,6 +61,9 @@ SIGNATURES = {
     "focusr_eigsort_workspace_bytes": (_sz, [_i, _i, _i, _i]),
     "focusr_eigsort_costs": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _i, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp,
                                   _vp, _sz, _vp]),
+    "focusr_eigsort_ragged_workspace_bytes": (_sz, [_vp, _vp, _i, _i]),
+    "focusr_eigsort_costs_ragged": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp,
+                                         _vp, _vp, _vp, _sz, _vp]),
     "focusr_eigsort_decide_workspace_bytes": (_sz, [_i, _i]),
     "focusr_eigsort_decide": (_i, [_vp, _i, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp,
                                    _vp, _sz, _vp]),

@@ -98,6 +98,25 @@ def check_icp_moving(mesh_pairs, target_to_source):
                                  m, "target" if target_to_source else "source", p, fixed[p], m, pairs.tolist()))
 
 
+def sample_indices_checked(idx, sizes, name):
+    """Checks user-supplied ordering samples of one side of a batch (``idx_t`` or ``idx_s``) against the sizes of that
+    side's meshes in pair order, and returns them in the form ``eigsort_costs`` takes (a 2-D array, or a list of 1-D
+    arrays).  ``ValueError`` unless there is one non-empty array of integers per pair, each in [0, size of its mesh)."""
+    if idx is None:
+        raise ValueError("give idx_t and idx_s together")
+    rows = _device.sample_rows(idx)
+    if len(rows) != len(sizes):
+        raise ValueError("%s needs one sample array per pair (%d), got %d" % (name, len(sizes), len(rows)))
+    for p, (r, sz) in enumerate(zip(rows, sizes)):
+        if r.size == 0:
+            raise ValueError("%s[%d] is empty: every pair needs at least one ordering sample" % (name, p))
+        lo, hi = int(r.min()), int(r.max())
+        if lo < 0 or hi >= sz:
+            raise ValueError("%s[%d] holds index %d outside [0, %d) (its mesh has %d vertices)" % (
+                name, p, lo if lo < 0 else hi, sz, sz))
+    return rows
+
+
 def layout_rows(src_off, mesh_of, dev):
     """A layout holding a copy of mesh ``mesh_of[i]`` of a batch with mesh offsets ``src_off`` (host), one after the
     other: its mesh offsets (host int32) and the batch row of every one of its rows (device int64)."""
@@ -240,8 +259,9 @@ class SpectralBatch:
 
     # ------------------------------------------------------------------------------------------
     def sample_indices(self, sizes, rng=None):
-        """Graph.get_list_rand_idxs (graph.py:274-290) for every mesh; all meshes must yield the
-        same count (n_samples <= every size, or n_samples > every size)."""
+        """Graph.get_list_rand_idxs (graph.py:274-290) for every mesh, in order: ``n_samples`` distinct rows of a mesh, or
+        all of its rows when it has fewer.  Returns a 2-D int64 array [len(sizes)][count] when every mesh yields the same
+        count, else a list of 1-D int64 arrays (``run`` and ``eigsort_costs`` take both)."""
         rng = rng or np.random.RandomState(self.seed)
         out = []
         for sz in sizes:
@@ -249,10 +269,9 @@ class SpectralBatch:
                 out.append(np.arange(sz, dtype=np.int64))
             else:
                 out.append(rng.choice(sz, size=self.n_samples, replace=False).astype(np.int64))
-        lens = {len(o) for o in out}
-        if len(lens) != 1:
-            raise ValueError("meshes of a batch must yield the same number of ordering samples")
-        return np.stack(out)
+        if len({len(o) for o in out}) == 1:
+            return np.stack(out)
+        return out
 
     # ------------------------------------------------------------------------------------------
     def run(self, points, tris, mesh_off_host, n_pairs, idx_t=None, idx_s=None, record_events=False,
@@ -304,6 +323,11 @@ class SpectralBatch:
             mp = mesh_pairs_checked(mesh_pairs, np.asarray(mesh_off_host).size - 1, P)
         if mp is not None and self.icp_register_first:
             check_icp_moving(mp, self.icp_reg_target_to_source)
+        if idx_t is not None:  # the pair layout's target and source sizes, from the host offsets
+            sizes = np.diff(np.asarray(mesh_off_host, dtype=np.int64))
+            t_sizes, s_sizes = (sizes[:P], sizes[P:2 * P]) if mp is None else (sizes[mp[:, 0]], sizes[mp[:, 1]])
+            idx_t = sample_indices_checked(idx_t, t_sizes, "idx_t")
+            idx_s = sample_indices_checked(idx_s, s_sizes, "idx_s")
         n_mesh_feats = len(self.list_features_to_get_from_mesh)
         if n_mesh_feats:
             n_total = int(np.asarray(mesh_off_host)[-1])
