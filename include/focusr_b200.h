@@ -473,6 +473,41 @@ int focusr_icp_batch(const double* points, int n_points, const int* tris, const 
                      double* moved_points, void* workspace, size_t workspace_bytes,
                      focusr_stream_t stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * K13  Statistical shape models (csrc/shape.cu): generalized Procrustes analysis and PCA of n_configs configurations
+ * [n_configs][n_points][3] (the n_points template vertices located on each subject), row-major, all device arrays.
+ * No call allocates, synchronises or reads anything back; every sum has a fixed order and none uses floating-point
+ * atomics, so repeated calls give the same bits.  Matrices are row-major 4x4 acting on column vectors, as focusr_icp's.
+ *
+ * focusr_procrustes_fit: for every configuration p, the vtkLandmarkTransform (rigid body, or similarity with scale
+ * sqrt(sum |ref - c_ref|^2 / sum |x - c_x|^2)) of configuration p onto `reference` [n_points][3] -- the fit of K10's
+ * iterations, by the same device code -- into mats_out [n_configs][16], and aligned_out [n_configs][n_points][3] =
+ * mats_out[p] * configuration p (nullable; must not alias `configs`).  A configuration's result depends only on it and
+ * the reference, not on the batch it is in.  n_points = 1 or coincident points give the identity rotation plus the
+ * translation of the centroids.
+ *
+ * focusr_procrustes_mean: the mean of `aligned` summed in p order and divided by n_configs, fitted onto `reference`
+ * (same mode) and transformed by that fit, into mean_out [n_points][3]; change_out (device, one double) =
+ * sqrt(sum_i |mean_out_i - prev_mean_i|^2 / n_points).  mean_out may be prev_mean.
+ *
+ * focusr_shape_gram: gram_out [n_configs][n_configs] = D D^T, D = aligned - mean (mean [n_points][3] subtracted from
+ * every configuration) viewed as [n_configs][3 n_points], on the FP64 tensor pipe; exactly symmetric.
+ *
+ * focusr_shape_modes: modes_out [n_modes][3 n_points] = D^T W for weights [n_configs][n_modes] (row-major), summed in
+ * configuration order.
+ * ------------------------------------------------------------------------------------------- */
+int focusr_procrustes_fit(const double* configs, int n_configs, int n_points, const double* reference, int similarity,
+                          double* mats_out, double* aligned_out, focusr_stream_t stream);
+size_t focusr_procrustes_mean_workspace_bytes(int n_points);
+int focusr_procrustes_mean(const double* aligned, int n_configs, int n_points, const double* reference, int similarity,
+                           const double* prev_mean, double* mean_out, double* change_out, void* workspace,
+                           size_t workspace_bytes, focusr_stream_t stream);
+size_t focusr_shape_gram_workspace_bytes(int n_configs, int n_points);
+int focusr_shape_gram(const double* aligned, const double* mean, int n_configs, int n_points, double* gram_out,
+                      void* workspace, size_t workspace_bytes, focusr_stream_t stream);
+int focusr_shape_modes(const double* aligned, const double* mean, int n_configs, int n_points, const double* weights,
+                       int n_modes, double* modes_out, focusr_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -454,6 +454,55 @@ def icp_batch(points, tris, mesh_off_host, tri_off_host, fixed_mesh, moving_mesh
     return mats.cpu().numpy(), moved
 
 
+def procrustes_fit(configs, reference, similarity, want_aligned=True):
+    """``focusr_procrustes_fit``: every configuration of ``configs`` (P, N, 3) fitted onto ``reference`` (N, 3), both
+    contiguous float64 device tensors.  Returns ``(matrices (P, 4, 4), aligned (P, N, 3) or None)`` on the device."""
+    torch = _torch()
+    P, N = int(configs.shape[0]), int(configs.shape[1])
+    mats = torch.empty((P, 4, 4), dtype=torch.float64, device=configs.device)
+    aligned = torch.empty_like(configs) if want_aligned else None
+    _lib.call("focusr_procrustes_fit", _lib.ptr(configs), P, N, _lib.ptr(reference), int(bool(similarity)), _lib.ptr(mats),
+              _lib.ptr(aligned), _lib.stream_ptr())
+    return mats, aligned
+
+
+def procrustes_mean(aligned, reference, similarity, prev_mean, mean_out, change_out, ws=None):
+    """``focusr_procrustes_mean``: the mean of ``aligned`` (P, N, 3) fitted onto ``reference`` into ``mean_out`` (N, 3),
+    its RMS change against ``prev_mean`` into ``change_out`` (a one-element device tensor).  ``ws``: a workspace of at
+    least ``focusr_procrustes_mean_workspace_bytes(N)`` bytes (allocated when None).  Returns the workspace."""
+    torch = _torch()
+    P, N = int(aligned.shape[0]), int(aligned.shape[1])
+    nbytes = int(_lib.load().focusr_procrustes_mean_workspace_bytes(N))
+    if ws is None or ws.numel() < nbytes:
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=aligned.device)
+    _lib.call("focusr_procrustes_mean", _lib.ptr(aligned), P, N, _lib.ptr(reference), int(bool(similarity)),
+              _lib.ptr(prev_mean), _lib.ptr(mean_out), _lib.ptr(change_out), _lib.ptr(ws), ws.numel(), _lib.stream_ptr())
+    return ws
+
+
+def shape_gram(aligned, mean):
+    """``focusr_shape_gram``: (P, P) float64 device tensor D D^T, D = ``aligned`` (P, N, 3) - ``mean`` (N, 3) as [P][3N]."""
+    torch = _torch()
+    P, N = int(aligned.shape[0]), int(aligned.shape[1])
+    nbytes = int(_lib.load().focusr_shape_gram_workspace_bytes(P, N))
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=aligned.device)
+    gram = torch.empty((P, P), dtype=torch.float64, device=aligned.device)
+    _lib.call("focusr_shape_gram", _lib.ptr(aligned), _lib.ptr(mean), P, N, _lib.ptr(gram), _lib.ptr(ws), nbytes,
+              _lib.stream_ptr())
+    return gram
+
+
+def shape_modes(aligned, mean, weights):
+    """``focusr_shape_modes``: (K, N, 3) float64 device tensor D^T W for ``weights`` (P, K), D as in :func:`shape_gram`."""
+    torch = _torch()
+    P, N, K = int(aligned.shape[0]), int(aligned.shape[1]), int(weights.shape[1])
+    w = weights.to(device=aligned.device, dtype=torch.float64).contiguous()
+    modes = torch.empty((K, N, 3), dtype=torch.float64, device=aligned.device)
+    _lib.call("focusr_shape_modes", _lib.ptr(aligned), _lib.ptr(mean), P, N, _lib.ptr(w), K, _lib.ptr(modes),
+              _lib.stream_ptr())
+    return modes
+
+
 def curvatures(points, tris):
     """vtkCurvatures on the device (vtk_functions.py:40-74).  ``points`` (N, 3) f64, ``tris`` (F, 3) i32, host or
     device.  Returns a dict of device tensors ``gauss``, ``mean``, ``minimum``, ``maximum``, each (N,)."""

@@ -92,6 +92,12 @@ SIGNATURES = {
     "focusr_cpd_kernel_matrix": (_i, [_vp, _i, _i, _d, _vp, _vp]),
     "focusr_cpd_affine_apply": (_i, [_vp, _i, _i, _vp, _vp, _vp, _vp]),
     "focusr_cpd_deformable_apply": (_i, [_vp, _i, _vp, _i, _i, _vp, _d, _vp, _vp]),
+    "focusr_procrustes_fit": (_i, [_vp, _i, _i, _vp, _i, _vp, _vp, _vp]),
+    "focusr_procrustes_mean_workspace_bytes": (_sz, [_i]),
+    "focusr_procrustes_mean": (_i, [_vp, _i, _i, _vp, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "focusr_shape_gram_workspace_bytes": (_sz, [_i, _i]),
+    "focusr_shape_gram": (_i, [_vp, _vp, _i, _i, _vp, _vp, _sz, _vp]),
+    "focusr_shape_modes": (_i, [_vp, _vp, _i, _i, _vp, _i, _vp, _vp]),
 }
 
 MESH_INFO_INTS = 8  # FOCUSR_MESH_INFO_INTS: {nnz, one-way entries, zero-degree rows, non-finite weights, longest row, ...}

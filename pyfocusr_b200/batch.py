@@ -828,3 +828,27 @@ class SpectralBatch:
         mp = mesh_pairs_checked(mesh_pairs, len(meshes))
         pts, tris, off = self._pack(meshes)
         return self._run_packed(meshes, pts, tris, off, mp.shape[0], dict(kw, mesh_pairs=mp))
+
+    def build_shape_model(self, subjects, template, rounds=5, template_tolerance=1e-3, procrustes="similarity",
+                          align_type="weighted", n_modes=10, **run_kw):
+        """A statistical shape model of the cohort ``subjects`` (PolyData-like meshes, any sizes) on the vertices of
+        ``template``.  Round k runs ``run_mesh_pairs(subjects + [template_k], [(m, P) for m in range(P)], **run_kw)`` with
+        this object's settings (the subjects are the targets, the template the shared source), takes the P
+        configurations [P][N_T][3] (every template vertex located on every subject) from
+        ``weighted_avg_transformed_points`` (``align_type="weighted"``) or ``nearest_neighbor_transformed_points``
+        (``"nearest"``), runs ``shape.procrustes`` on them (``procrustes``: "rigid" or "similarity") with template_k's
+        points as the reference, and makes template_{k+1} = the GPA mean on the template's triangles.  Rounds stop when
+        RMS(template_{k+1} - template_k) <= ``template_tolerance`` (in the units of the points) or after ``rounds``;
+        ``shape.pca`` then runs on the last round's aligned configurations.
+
+        Returns a dict: ``mean_points`` (N_T, 3) and ``mean_mesh`` (the last template_{k+1}); ``aligned`` (P, N_T, 3) and
+        ``procrustes_matrices`` (P, 4, 4) of the last GPA; ``modes``, ``variances``, ``scores`` of ``shape.pca`` with
+        ``n_modes``; ``rounds``, one dict per round with ``template_change``, ``gpa_iterations``, ``gpa_changes`` and,
+        with ICP on, ``icp_matrices``.  ``ValueError`` before any device work for no subjects, a bad ``procrustes`` or
+        ``align_type``, ``n_modes`` < 1, ``rounds`` < 1, or ``icp_register_first`` without ``icp_reg_target_to_source``
+        (the shared template would be every pair's moving mesh).  A failed registration (an eigensolve, a zero-length
+        edge in an averaged template) raises ``RuntimeError`` naming the round and the subjects or template."""
+        from .shape import build_shape_model
+
+        return build_shape_model(self, subjects, template, rounds=rounds, template_tolerance=template_tolerance,
+                                 procrustes_mode=procrustes, align_type=align_type, n_modes=n_modes, **run_kw)

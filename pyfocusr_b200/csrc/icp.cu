@@ -37,6 +37,7 @@
 #include <cub/device/device_segmented_radix_sort.cuh>
 
 #include "common.cuh"
+#include "landmark_fit.cuh"
 #include "morton.cuh"
 
 namespace fb {
@@ -91,18 +92,6 @@ __device__ __forceinline__ P3 closest_on_triangle(P3 p, P3 a, P3 b, P3 c) {
 __device__ __forceinline__ P3 xform(const double* __restrict__ m, P3 p) {  // 4x4 row-major, column vectors
   return P3{m[0] * p.x + m[1] * p.y + m[2] * p.z + m[3], m[4] * p.x + m[5] * p.y + m[6] * p.z + m[7],
             m[8] * p.x + m[9] * p.y + m[10] * p.z + m[11]};
-}
-
-__device__ __forceinline__ double icp_block_sum(double v, double* red) {
-  const int t = threadIdx.x;
-  __syncthreads();
-  red[t] = v;
-  __syncthreads();
-  for (int s = blockDim.x >> 1; s > 0; s >>= 1) {
-    if (t < s) red[t] += red[t + s];
-    __syncthreads();
-  }
-  return red[0];
 }
 
 // one (fixed, moving) pair; point indices are rows of the call's fixed / moving point arrays
@@ -195,7 +184,7 @@ __global__ void __launch_bounds__(1024) k_icp_start(const IcpPair* __restrict__ 
   }
   double tr[3];
   for (int d = 0; d < 3; ++d) {
-    const double a = icp_block_sum(s[d], red), b = icp_block_sum(g[d], red);
+    const double a = fit_block_sum(s[d], red), b = fit_block_sum(g[d], red);
     tr[d] = match ? b / nt - a / ns : 0.0;
   }
   if (threadIdx.x == 0) {
@@ -541,114 +530,15 @@ k_icp_closest(const IcpPair* __restrict__ pairs, int P, const int* __restrict__ 
 }
 
 // vtkLandmarkTransform (rigid body / similarity) of a -> b, then acc <- L * acc; one CTA per pair
-__global__ void __launch_bounds__(256) k_icp_fit(const int* __restrict__ off_lm, const double* __restrict__ a_all,
-                                                const double* __restrict__ b_all, int similarity, double* __restrict__ L_all,
-                                                double* __restrict__ acc_all) {
-  __shared__ double red[256];
+__global__ void __launch_bounds__(FIT_THREADS) k_icp_fit(const int* __restrict__ off_lm, const double* __restrict__ a_all,
+                                                        const double* __restrict__ b_all, int similarity, double* __restrict__ L_all,
+                                                        double* __restrict__ acc_all) {
+  __shared__ double red[FIT_THREADS];
   const int l0 = off_lm[blockIdx.x], nb = off_lm[blockIdx.x + 1] - l0;
-  const double* a = a_all + 3 * (size_t)l0;
-  const double* b = b_all + 3 * (size_t)l0;
   double* L = L_all + 16 * (size_t)blockIdx.x;
   double* acc = acc_all + 16 * (size_t)blockIdx.x;
-  const int t = threadIdx.x;
-  double s[6] = {0, 0, 0, 0, 0, 0};
-  for (int i = t; i < nb; i += 256)
-    for (int d = 0; d < 3; ++d) {
-      s[d] += a[3 * i + d];
-      s[3 + d] += b[3 * i + d];
-    }
-  double ca[3], cb[3];
-  for (int d = 0; d < 3; ++d) {
-    ca[d] = icp_block_sum(s[d], red) / nb;
-    cb[d] = icp_block_sum(s[3 + d], red) / nb;
-  }
-  double m[11] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};  // M row-major, sa, sb
-  for (int i = t; i < nb; i += 256) {
-    double x[3], y[3];
-    for (int d = 0; d < 3; ++d) {
-      x[d] = a[3 * i + d] - ca[d];
-      y[d] = b[3 * i + d] - cb[d];
-    }
-    for (int r = 0; r < 3; ++r)
-      for (int c = 0; c < 3; ++c) m[3 * r + c] += x[r] * y[c];
-    m[9] += x[0] * x[0] + x[1] * x[1] + x[2] * x[2];
-    m[10] += y[0] * y[0] + y[1] * y[1] + y[2] * y[2];
-  }
-  double M[11];
-  for (int k = 0; k < 11; ++k) M[k] = icp_block_sum(m[k], red);
-  if (t != 0) return;
-  double R[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1};
-  const double sa = M[9], sb = M[10];
-  if (nb > 1 && sa != 0.0 && sb != 0.0) {
-    double N[4][4], V[4][4];
-    N[0][0] = M[0] + M[4] + M[8];
-    N[1][1] = M[0] - M[4] - M[8];
-    N[2][2] = -M[0] + M[4] - M[8];
-    N[3][3] = -M[0] - M[4] + M[8];
-    N[0][1] = N[1][0] = M[5] - M[7];
-    N[0][2] = N[2][0] = M[6] - M[2];
-    N[0][3] = N[3][0] = M[1] - M[3];
-    N[1][2] = N[2][1] = M[1] + M[3];
-    N[1][3] = N[3][1] = M[6] + M[2];
-    N[2][3] = N[3][2] = M[5] + M[7];
-    for (int i = 0; i < 4; ++i)
-      for (int j = 0; j < 4; ++j) V[i][j] = i == j ? 1.0 : 0.0;
-    for (int sweep = 0; sweep < 60; ++sweep) {  // cyclic Jacobi
-      double off = 0.0, diag = 0.0;
-      for (int i = 0; i < 4; ++i) {
-        diag += N[i][i] * N[i][i];
-        for (int j = i + 1; j < 4; ++j) off += N[i][j] * N[i][j];
-      }
-      if (off <= 1e-32 * diag || off == 0.0) break;
-      for (int p = 0; p < 3; ++p)
-        for (int q = p + 1; q < 4; ++q) {
-          if (N[p][q] == 0.0) continue;
-          const double theta = (N[q][q] - N[p][p]) / (2.0 * N[p][q]);
-          const double tt = (theta >= 0.0 ? 1.0 : -1.0) / (fabs(theta) + sqrt(theta * theta + 1.0));
-          const double c = 1.0 / sqrt(tt * tt + 1.0), sn = tt * c;
-          for (int k = 0; k < 4; ++k) {
-            const double nkp = N[k][p], nkq = N[k][q];
-            N[k][p] = c * nkp - sn * nkq;
-            N[k][q] = sn * nkp + c * nkq;
-          }
-          for (int k = 0; k < 4; ++k) {
-            const double npk = N[p][k], nqk = N[q][k];
-            N[p][k] = c * npk - sn * nqk;
-            N[q][k] = sn * npk + c * nqk;
-          }
-          for (int k = 0; k < 4; ++k) {
-            const double vkp = V[k][p], vkq = V[k][q];
-            V[k][p] = c * vkp - sn * vkq;
-            V[k][q] = sn * vkp + c * vkq;
-          }
-        }
-    }
-    int top = 0;
-    for (int i = 1; i < 4; ++i)
-      if (N[i][i] > N[top][top]) top = i;
-    const double w = V[0][top], x = V[1][top], y = V[2][top], z = V[3][top];
-    const double ww = w * w, wx = w * x, wy = w * y, wz = w * z, xx = x * x, yy = y * y, zz = z * z, xy = x * y, xz = x * z, yz = y * z;
-    R[0] = ww + xx - yy - zz;
-    R[3] = 2.0 * (wz + xy);
-    R[6] = 2.0 * (-wy + xz);
-    R[1] = 2.0 * (-wz + xy);
-    R[4] = ww - xx + yy - zz;
-    R[7] = 2.0 * (wx + yz);
-    R[2] = 2.0 * (wy + xz);
-    R[5] = 2.0 * (-wx + yz);
-    R[8] = ww - xx - yy + zz;
-    if (similarity) {
-      const double sc = sqrt(sb / sa);
-      for (int i = 0; i < 9; ++i) R[i] *= sc;
-    }
-  }
   double Lm[16];
-  for (int r = 0; r < 3; ++r) {
-    for (int c = 0; c < 3; ++c) Lm[4 * r + c] = R[3 * r + c];
-    Lm[4 * r + 3] = cb[r] - (R[3 * r] * ca[0] + R[3 * r + 1] * ca[1] + R[3 * r + 2] * ca[2]);
-  }
-  Lm[12] = Lm[13] = Lm[14] = 0.0;
-  Lm[15] = 1.0;
+  if (!landmark_fit_block(a_all + 3 * (size_t)l0, b_all + 3 * (size_t)l0, nb, similarity, red, Lm)) return;
   double old[16], nw[16];
   for (int i = 0; i < 16; ++i) old[i] = acc[i];
   for (int r = 0; r < 4; ++r)
@@ -840,7 +730,7 @@ static int icp_run(const IcpSizes& s, void* workspace, size_t workspace_bytes, c
     k_icp_closest<<<div_up(n_groups, ICP_WARPS), 32 * ICP_WARPS, 0, stream>>>(
         w.pairs, P, w.off_lm, w.off_grp, w.off_tri, w.off_tile, group, n_groups, w.box, w.tv, w.tid, w.tile_lo, w.tile_hi,
         w.tile_key, w.perm, w.a, it > 0 ? 1 : 0, w.winner, w.cl);
-    k_icp_fit<<<P, 256, 0, stream>>>(w.off_lm, w.a, w.cl, similarity ? 1 : 0, L, acc);
+    k_icp_fit<<<P, FIT_THREADS, 0, stream>>>(w.off_lm, w.a, w.cl, similarity ? 1 : 0, L, acc);
     FB_COUNT_LAUNCH(2);
     if (it + 1 >= max_iterations) break;
     k_icp_move<<<g_lm, 256, 0, stream>>>(w.off_lm, L, w.a);
