@@ -215,7 +215,9 @@ int focusr_eigs_smallest_dist(const int* row_ptr, const int* cols_local, const d
  * row-partitioned solve of this process: {nanoseconds CTA 0 spent at the in-kernel barriers, nanoseconds it spent
  * working, steps, 0}.  kind 4 = the pruned KNN: {(query, reference) distance evaluations since the last reset, 0, 0,
  * 0} (synchronises the device).  kind 5 = the ICP closest-point search: {(landmark, triangle) evaluations since the last
- * reset, 0, 0, 0}, counted only by a build with -DFB_ICP_COUNT (0 otherwise; synchronises the device). */
+ * reset, 0, 0, 0}, counted only by a build with -DFB_ICP_COUNT (0 otherwise; synchronises the device).  kind 6 = the
+ * pruned surface closest-point search (focusr_closest_points): {(query, triangle) evaluations since the last reset, the
+ * home-tile seeds included, 0, 0, 0}, counted only by a build with -DFB_SURFACE_COUNT (0 otherwise; synchronises). */
 void focusr_profile_reset(void);
 void focusr_profile_get(double* out4_host);
 void focusr_profile_get_kind(int kind, double* out4_host);
@@ -507,6 +509,46 @@ int focusr_shape_gram(const double* aligned, const double* mean, int n_configs, 
                       void* workspace, size_t workspace_bytes, focusr_stream_t stream);
 int focusr_shape_modes(const double* aligned, const double* mean, int n_configs, int n_points, const double* weights,
                        int n_modes, double* modes_out, focusr_stream_t stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * K14  Surface distances (csrc/surface.cu): the closest point on a triangle surface of every query point, and per pair
+ * the summary of two such searches (source -> target surface and target -> source surface).
+ *
+ * focusr_closest_points: surfaces in the batch layout (`tris` [..][3] with global vertex ids into `surf_points`
+ * [..][3]; surface m = points surf_point_off[m] .. [m+1], triangles surf_tri_off[m] .. [m+1]); query segment s =
+ * queries[query_off[s] .. query_off[s+1]) ([..][3]), searched against surface surf_of_segment[s].  A surface may serve
+ * several segments, one or none; empty segments are allowed.  Outputs, indexed like `queries`, each nullable:
+ * closest_out [..][3] the closest point on the surface, tri_out [..] the winning triangle as an index local to its
+ * surface's triangle range, dist_out [..] the Euclidean distance.  The winner is the lexicographic minimum of (d^2, local
+ * triangle index) over every triangle of the surface, each scored by Ericson's region test (the arithmetic of K10's
+ * search); a triangle whose region solve would divide by zero (collapsed to a segment or a point: va + vb + vc == 0, or
+ * a zero-length edge) is scored as the closest of its edges ab, bc, ca, a tie keeping the earlier edge and a zero-length
+ * edge scoring as its end point.  workspace = NULL selects a plain scan of every triangle in index order; with a
+ * workspace (focusr_closest_points_workspace_bytes) each mapped surface is Morton-sorted and cut into tiles of 32
+ * triangles once, and each warp of 32 Morton-grouped queries visits only the tiles within its group's bound: same
+ * arithmetic, bit-identical output.  The `_host` arrays are host copies of the device arrays of the same name.  It is
+ * an argument error, and the workspace size is 0, when there is no surface or no segment, an offset table is negative
+ * or not monotone, a surface index is out of range, or a mapped surface has no triangles.  Triangle ids must lie in
+ * range: the call does not check them.  A segment's results depend only on its queries and its surface: not on the
+ * batch, nor on how many segments share the surface.
+ *
+ * focusr_surface_distance_stats: per pair p, stats_out [n_pairs][6] = {mean a->b, max a->b, mean b->a, max b->a,
+ * ASSD = (sum a->b + sum b->a) / (n_a + n_b), Hausdorff = max of the two maxima}, from the per-query distances a_dist
+ * [a_off[p] .. a_off[p+1]) and b_dist [b_off[p] .. b_off[p+1]) (device offsets).  A side without distances has NaN mean
+ * and max, and the pair a NaN Hausdorff distance.  One CTA per pair, sums in a fixed order.
+ *
+ * Neither call allocates, synchronises or reads anything back, and neither uses floating-point atomics: two calls give
+ * the same bits.
+ * ------------------------------------------------------------------------------------------- */
+size_t focusr_closest_points_workspace_bytes(const int* surf_point_off_host, const int* surf_tri_off_host, int n_surfaces,
+                                             const int* query_off_host, int n_segments, const int* surf_of_segment_host);
+int focusr_closest_points(const double* surf_points, const int* tris, const int* surf_point_off, const int* surf_tri_off,
+                          const int* surf_point_off_host, const int* surf_tri_off_host, int n_surfaces,
+                          const double* queries, const int* query_off, const int* query_off_host, int n_segments,
+                          const int* surf_of_segment, const int* surf_of_segment_host, double* closest_out, int* tri_out,
+                          double* dist_out, void* workspace, size_t workspace_bytes, focusr_stream_t stream);
+int focusr_surface_distance_stats(const double* a_dist, const int* a_off, const double* b_dist, const int* b_off,
+                                  int n_pairs, double* stats_out, focusr_stream_t stream);
 
 #ifdef __cplusplus
 }

@@ -12,9 +12,10 @@ from .eigsort import eigsort
 from .focusr import Focusr
 from .graph import Graph, recursive_eig
 from .mesh import PolyData, ellipsoid_pair, icosphere, perturbed_ellipsoid, read_vtk_mesh, write_vtk_mesh
+from .surface import surface_distances
 
 __all__ = [
     "Focusr", "Graph", "recursive_eig", "eigsort", "SpectralBatch", "PolyData", "read_vtk_mesh", "write_vtk_mesh",
-    "icosphere", "perturbed_ellipsoid", "ellipsoid_pair", "vtk_functions",
+    "icosphere", "perturbed_ellipsoid", "ellipsoid_pair", "vtk_functions", "surface_distances",
 ]
 __version__ = "0.1.0"

@@ -98,6 +98,9 @@ SIGNATURES = {
     "focusr_shape_gram_workspace_bytes": (_sz, [_i, _i]),
     "focusr_shape_gram": (_i, [_vp, _vp, _i, _i, _vp, _vp, _sz, _vp]),
     "focusr_shape_modes": (_i, [_vp, _vp, _i, _i, _vp, _i, _vp, _vp]),
+    "focusr_closest_points_workspace_bytes": (_sz, [_vp, _vp, _i, _vp, _i, _vp]),
+    "focusr_closest_points": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "focusr_surface_distance_stats": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _vp]),
 }
 
 MESH_INFO_INTS = 8  # FOCUSR_MESH_INFO_INTS: {nnz, one-way entries, zero-degree rows, non-finite weights, longest row, ...}

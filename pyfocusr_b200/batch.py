@@ -27,12 +27,16 @@ import numpy as np
 
 from . import _device, _lib
 from ._device import DeviceGraph
+from .shape import ALIGN_TYPES
 
 __all__ = ["SpectralBatch"]
 
 # graph.py:11-15 (features_dictionary): the focusr_curvatures outputs each name contributes, in order
 CURVATURE_FEATURES = {"curvature": ("minimum", "maximum"), "min_curvature": ("minimum",), "max_curvature": ("maximum",)}
 MAX_KNN_DIM, MAX_CPD_DIM = 32, 16  # focusr_knn, focusr_cpd_*
+# SpectralBatch(surface_distances=...): the transformed source positions whose surface is measured, by the names of
+# build_shape_model's align_type
+SURFACE_POSITIONS = ALIGN_TYPES
 
 
 def shared_targets(target_of_pair, n_meshes, n_pairs):
@@ -185,7 +189,18 @@ class SpectralBatch:
                  icp_reg_target_to_source=False, list_features_to_calc=("curvature",), list_features_to_get_from_mesh=(),
                  include_features_in_adj_matrix=False, use_features_as_coords=False, feature_smoothing_iterations=40,
                  norm_node_features_std=True, norm_node_features_cap_std=3, norm_node_features_0_1=True,
-                 include_points_as_features=False, norm_physical_and_spectral=True):
+                 include_points_as_features=False, norm_physical_and_spectral=True, surface_distances=None):
+        """The keyword names and defaults of ``Focusr`` where the two share a setting.  ``surface_distances``: None (the
+        default: no extra work, no extra keys), or ``"weighted"`` / ``"nearest"`` to have ``run`` measure, for every
+        pair, the distances between its transformed source (``weighted_avg_transformed_points`` or
+        ``nearest_neighbor_transformed_points`` on the source mesh's triangles) and its target surface, both ways.  The
+        keys this adds to ``run``'s result: ``source_to_target_surface_dist``, ``source_to_target_closest_points``,
+        ``source_to_target_closest_tri``, ``target_to_source_surface_dist``, ``target_to_source_closest_tri`` and
+        ``surface_distance_stats`` (see ``run``); ``build_shape_model`` then reports ``surface_distance_stats`` per
+        round.  ``ValueError`` for any other value."""
+        if surface_distances is not None and not (isinstance(surface_distances, str) and surface_distances in SURFACE_POSITIONS):
+            raise ValueError("surface_distances must be None, 'weighted' or 'nearest', got %r" % (surface_distances,))
+        self.surface_distances = surface_distances
         self.ns = int(n_spectral_features)
         self.n = int(n_spectral_features + n_extra_spectral)
         self.n_samples = int(n_coords_spectral_ordering)
@@ -308,7 +323,19 @@ class SpectralBatch:
         in mesh_pairs])``), except ``graph`` and ``eigs_info``, which describe the M meshes; ``pair_mesh_off`` holds the
         pair layout's offsets.  ``ValueError`` for a malformed list, a mesh outside [0, M) or used by no pair, ``n_pairs
         != P``, ``target_of_pair`` given too, or, with ICP on, a moving mesh that is not in exactly one pair or is that
-        pair's fixed mesh.  ``target_of_pair`` is the case ``mesh_pairs = [(target_of_pair[p], T + p)]``."""
+        pair's fixed mesh.  ``target_of_pair`` is the case ``mesh_pairs = [(target_of_pair[p], T + p)]``.
+
+        With ``surface_distances`` set (``SpectralBatch(surface_distances="weighted" | "nearest")``) the result gains, on
+        the rows of the pair layout: ``source_to_target_surface_dist`` [source rows] (each transformed source vertex to
+        its pair's target surface: the batch graph's target points, after ICP when it is on, and triangles),
+        ``source_to_target_closest_points`` [source rows][3] (the point on that surface), ``source_to_target_closest_tri``
+        [source rows] int64 (the triangle, local to the target mesh), ``target_to_source_surface_dist`` [target rows]
+        (each target vertex to its pair's transformed source surface: the source mesh's triangles on the pair's
+        transformed positions), ``target_to_source_closest_tri`` [target rows] int64 (local to the source mesh) and
+        ``surface_distance_stats`` (P, 6) (mean and max source -> target, mean and max target -> source, ASSD, Hausdorff;
+        ``surface.STATS_COLUMNS``).  The triangle ranges come from ``tri_off_host``, or from ``tris`` as for ICP.  Every
+        other key is unchanged, and with shared meshes every new key equals that of the repeated-mesh batch, bit for
+        bit.  ``record_events`` then times a ``surface`` stage."""
         P = int(n_pairs)
         mp = None  # (target mesh, source mesh) of every pair when meshes are shared, else None (mesh p with mesh P + p)
         if target_of_pair is not None and mesh_pairs is not None:
@@ -494,6 +521,11 @@ class SpectralBatch:
             smoothed_tc = _device.gather_rows(smoothed_t, layout_rows(tb.mesh_off_host, cb_of, dev)[1])
             if feats is not None:
                 feats = pg.rows(feats)
+        surf = {}
+        if self.surface_distances is not None:
+            positions = weighted if self.surface_distances == "weighted" else nearest
+            surf = self._surface(g, pg, positions, tri_off_host, mp, P)
+            mark("surface")
         if record_events:
             torch.cuda.synchronize()
             self.timings = {ev[i][0]: ev[i - 1][1].elapsed_time(ev[i][1]) for i in range(1, len(ev))}
@@ -504,7 +536,41 @@ class SpectralBatch:
                     knn3_dist=dist3, weighted_avg_transformed_points=weighted,
                     nearest_neighbor_transformed_points=nearest, idx_t=idx_t, idx_s=idx_s, costs=costs,
                     eig_vecs_presort=presort, cpd_idx=cpd_idx, coords_b4_reg=coords_b4_reg, icp_matrices=icp_mats,
-                    node_features=feats)
+                    node_features=feats, **surf)
+
+    def _surface(self, g, pg, positions, tri_off_host, mesh_pairs, P):
+        """The surface-distance keys of ``run``: every pair's transformed source rows (``positions``, the source rows of
+        the pair layout ``pg``) against its target mesh of the batch graph ``g`` (each distinct target tiled once), and
+        the pair layout's target rows against the pair's source triangles re-based onto the pair's rows of
+        ``positions``."""
+        from . import surface
+
+        torch = _lib.require_cuda()
+        dev = g.device
+        if tri_off_host is None:
+            tri_off = self.tri_offsets(g.tris, g.mesh_off_host)
+        else:
+            tri_off = np.ascontiguousarray(tri_off_host, dtype=np.int32).reshape(-1)
+            if tri_off.size != g.n_meshes + 1 or tri_off[0] != 0 or tri_off[-1] != g.n_tris or np.any(np.diff(tri_off) < 0):
+                raise ValueError("tri_off_host must hold %d non-decreasing triangle offsets from 0 to %d" % (
+                    g.n_meshes + 1, g.n_tris))
+        t_mesh, s_mesh = (np.arange(P), np.arange(P, 2 * P)) if mesh_pairs is None else (mesh_pairs[:, 0], mesh_pairs[:, 1])
+        off = pg.mesh_off_host
+        nt_pair = int(off[P])
+        src_off, tgt_off = (off[P:] - nt_pair).astype(np.int32), off[:P + 1]
+        closest, s_tri, s_dist = surface.closest_points(g.points, g.tris, g.mesh_off_host, tri_off, positions, src_off, t_mesh)
+        # pair p's source triangles, their ids moved from the source mesh's rows of g to pair p's rows of `positions`
+        s_tri_off, tri_rows = layout_rows(tri_off, s_mesh, dev)
+        shift = torch.from_numpy(src_off[:-1].astype(np.int64) - g.mesh_off_host[s_mesh]).to(dev, non_blocking=True)
+        shift = torch.repeat_interleave(shift, torch.from_numpy(np.diff(s_tri_off).astype(np.int64)).to(dev, non_blocking=True),
+                                        output_size=int(s_tri_off[-1]))
+        s_tris = (g.tris.index_select(0, tri_rows) + shift[:, None]).to(torch.int32).contiguous()
+        _, t_tri, t_dist = surface.closest_points(positions, s_tris, src_off, s_tri_off, pg.points[:nt_pair], tgt_off,
+                                                  np.arange(P), want_closest=False)
+        return dict(source_to_target_surface_dist=s_dist, source_to_target_closest_points=closest,
+                    source_to_target_closest_tri=s_tri, target_to_source_surface_dist=t_dist,
+                    target_to_source_closest_tri=t_tri,
+                    surface_distance_stats=surface.distance_stats(s_dist, src_off, t_dist, tgt_off))
 
     @staticmethod
     def _mesh_pairs(m, mesh_pairs):
@@ -843,8 +909,9 @@ class SpectralBatch:
 
         Returns a dict: ``mean_points`` (N_T, 3) and ``mean_mesh`` (the last template_{k+1}); ``aligned`` (P, N_T, 3) and
         ``procrustes_matrices`` (P, 4, 4) of the last GPA; ``modes``, ``variances``, ``scores`` of ``shape.pca`` with
-        ``n_modes``; ``rounds``, one dict per round with ``template_change``, ``gpa_iterations``, ``gpa_changes`` and,
-        with ICP on, ``icp_matrices``.  ``ValueError`` before any device work for no subjects, a bad ``procrustes`` or
+        ``n_modes``; ``rounds``, one dict per round with ``template_change``, ``gpa_iterations``, ``gpa_changes``,
+        with ICP on ``icp_matrices`` and, with ``surface_distances`` set, ``surface_distance_stats`` ((P, 6) host numpy,
+        row m for subject m: the template is the source).  ``ValueError`` before any device work for no subjects, a bad ``procrustes`` or
         ``align_type``, ``n_modes`` < 1, ``rounds`` < 1, or ``icp_register_first`` without ``icp_reg_target_to_source``
         (the shared template would be every pair's moving mesh).  A failed registration (an eigensolve, a zero-length
         edge in an averaged template) raises ``RuntimeError`` naming the round and the subjects or template."""

@@ -24,6 +24,8 @@ namespace fb {
 
 unsigned long long pk_evals_read_and_maybe_reset(bool reset);  // knn_pruned.cu
 unsigned long long icp_evals_read_and_maybe_reset(bool reset);  // icp.cu
+// surface.cu; weak, so that a library linking this file without surface.cu (tests/kernel_probe) still loads
+unsigned long long surface_evals_read_and_maybe_reset(bool reset) __attribute__((weak));
 
 constexpr int GRAM_ROWS = 1024;  // rows per CTA (8 warps x 128 rows)
 constexpr int GRAM_THREADS = 256;
@@ -1346,6 +1348,7 @@ extern "C" {
 void focusr_profile_reset(void) {
   pk_evals_read_and_maybe_reset(true);
   icp_evals_read_and_maybe_reset(true);
+  if (surface_evals_read_and_maybe_reset) surface_evals_read_and_maybe_reset(true);
   g_filter_profile.collect();
   g_filter_profile_lowp.collect();
   g_filter_profile_corr.collect();
@@ -1366,6 +1369,13 @@ void focusr_profile_get_kind(int kind, double* out4_host) {
                     // builds with -DFB_ICP_COUNT (synchronises the device)
     cudaDeviceSynchronize();
     out4_host[0] = (double)icp_evals_read_and_maybe_reset(false);
+    out4_host[1] = out4_host[2] = out4_host[3] = 0.0;
+    return;
+  }
+  if (kind == 6) {  // surface closest-point search: (query, triangle) evaluations since the last reset, counted only in
+                    // builds with -DFB_SURFACE_COUNT (synchronises the device)
+    cudaDeviceSynchronize();
+    out4_host[0] = surface_evals_read_and_maybe_reset ? (double)surface_evals_read_and_maybe_reset(false) : 0.0;
     out4_host[1] = out4_host[2] = out4_host[3] = 0.0;
     return;
   }

@@ -36,6 +36,7 @@
 
 #include <cub/device/device_segmented_radix_sort.cuh>
 
+#include "closest_point.cuh"
 #include "common.cuh"
 #include "landmark_fit.cuh"
 #include "morton.cuh"
@@ -58,36 +59,6 @@ constexpr int ICP_WARPS = 4;   // groups per CTA of k_icp_closest
 // sort reads segment sizes back to the host for batches of more than 500 segments).
 constexpr int ICP_SORT_BITS[2] = {32, 62};
 constexpr int ICP_BOX = 8;     // doubles per (pair, mesh) box record: lo[3], 1024 / extent[3], pad, 0
-
-struct P3 {
-  double x, y, z;
-};
-__device__ __forceinline__ P3 p3(const double* __restrict__ p, long long i) { return P3{p[3 * i], p[3 * i + 1], p[3 * i + 2]}; }
-__device__ __forceinline__ P3 operator-(P3 a, P3 b) { return P3{a.x - b.x, a.y - b.y, a.z - b.z}; }
-__device__ __forceinline__ P3 operator+(P3 a, P3 b) { return P3{a.x + b.x, a.y + b.y, a.z + b.z}; }
-__device__ __forceinline__ P3 operator*(P3 a, double s) { return P3{a.x * s, a.y * s, a.z * s}; }
-__device__ __forceinline__ double dot3(P3 a, P3 b) { return a.x * b.x + a.y * b.y + a.z * b.z; }
-
-// closest point of triangle (a, b, c) to p: Ericson, "Real-Time Collision Detection", 5.1.5
-__device__ __forceinline__ P3 closest_on_triangle(P3 p, P3 a, P3 b, P3 c) {
-  const P3 ab = b - a, ac = c - a, ap = p - a;
-  const double d1 = dot3(ab, ap), d2 = dot3(ac, ap);
-  if (d1 <= 0.0 && d2 <= 0.0) return a;
-  const P3 bp = p - b;
-  const double d3 = dot3(ab, bp), d4 = dot3(ac, bp);
-  if (d3 >= 0.0 && d4 <= d3) return b;
-  const double vc = d1 * d4 - d3 * d2;
-  if (vc <= 0.0 && d1 >= 0.0 && d3 <= 0.0) return a + ab * (d1 / (d1 - d3));
-  const P3 cp = p - c;
-  const double d5 = dot3(ab, cp), d6 = dot3(ac, cp);
-  if (d6 >= 0.0 && d5 <= d6) return c;
-  const double vb = d5 * d2 - d1 * d6;
-  if (vb <= 0.0 && d2 >= 0.0 && d6 <= 0.0) return a + ac * (d2 / (d2 - d6));
-  const double va = d3 * d6 - d5 * d4;
-  if (va <= 0.0 && (d4 - d3) >= 0.0 && (d5 - d6) >= 0.0) return b + (c - b) * ((d4 - d3) / ((d4 - d3) + (d5 - d6)));
-  const double denom = 1.0 / (va + vb + vc);
-  return a + ab * (vb * denom) + ac * (vc * denom);
-}
 
 __device__ __forceinline__ P3 xform(const double* __restrict__ m, P3 p) {  // 4x4 row-major, column vectors
   return P3{m[0] * p.x + m[1] * p.y + m[2] * p.z + m[3], m[4] * p.x + m[5] * p.y + m[6] * p.z + m[7],
@@ -316,14 +287,6 @@ __global__ void k_icp_init_landmarks(const IcpPair* __restrict__ pairs, const in
   a[3 * i] = q.x;
   a[3 * i + 1] = q.y;
   a[3 * i + 2] = q.z;
-}
-
-// squared distance from q to an axis-aligned box, rounded down
-__device__ __forceinline__ double box_lb(P3 q, const double* __restrict__ lo, const double* __restrict__ hi) {
-  const double g0 = fmax(fmax(lo[0] - q.x, q.x - hi[0]), 0.0);
-  const double g1 = fmax(fmax(lo[1] - q.y, q.y - hi[1]), 0.0);
-  const double g2 = fmax(fmax(lo[2] - q.z, q.z - hi[2]), 0.0);
-  return (g0 * g0 + g1 * g1 + g2 * g2) * (1.0 - 1e-12);
 }
 
 // (landmark, triangle) closest-point evaluations of k_icp_closest since the last reset; counted only in builds with

@@ -160,6 +160,8 @@ def build_shape_model(sb, subjects, template, rounds=5, template_tolerance=1e-3,
         info = dict(template_change=change, gpa_iterations=gpa["iterations"], gpa_changes=gpa["changes"])
         if sb.icp_register_first:
             info["icp_matrices"] = out["icp_matrices"]
+        if sb.surface_distances is not None:  # the template is every pair's source: one row per subject
+            info["surface_distance_stats"] = out["surface_distance_stats"].cpu().numpy()
         per_round.append(info)
         del out, configs
         tmpl = PolyData(new_points, template.tris, getattr(template, "point_scalars", None))
